@@ -1,8 +1,11 @@
 #!/usr/bin/env python3
 """bench.py - NMF restart-iterations/sec of the B200-native NMFk hot path.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--config auto|C2|C3|C4|C5]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--config auto|C2|C3|C4|C5] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
+
+--dump-outputs DIR writes what the timed GPU path returned in its last timed step as DIR/<name>.npy (see dump_outputs): the
+inputs are seeded, so two builds run with the same arguments can be compared output for output.
 
 Workloads (BASELINE.json `configs`, SURVEY.md 8(d); synthetic nonnegative mixtures X = W0*H0, seed 2015):
   N = 1 (default)  C3: 10000 x 10000 Float32, k = 16, nNMF = 64 - the largest single-GPU configuration.  One step = ITERS
@@ -38,7 +41,9 @@ import subprocess  # noqa: E402
 import sys  # noqa: E402
 import threading  # noqa: E402
 import time  # noqa: E402
+import zlib  # noqa: E402
 
+sys.dont_write_bytecode = True  # the benchmark writes nothing into the tree it runs from (which may be read-only)
 ROOT = os.path.dirname(os.path.abspath(__file__))
 for p in (ROOT, os.path.join(ROOT, "nmfk.jl_b200", "python")):
     if p not in sys.path:
@@ -124,6 +129,25 @@ class ClockSampler:
                 pass
         return {"sm_mhz": statistics.median(sm) if sm else None, "sm_max_mhz": max(smax) if smax else None,
                 "reasons": sorted(reasons), "samples": len(sm)}
+
+
+DUMP_BYTES = 60 << 20  # data written by --dump-outputs in all: below 64 MB with the .npy headers
+BATCH_FIELDS = ("W", "H", "obj_ssq", "obj_norm", "iters", "stop_reason")  # what Batch.get returns for a solved batch
+
+
+def dump_outputs(path, arrays):
+    """Writes every entry of `arrays` as path/<name>.npy: Float32 arrays as Float32, everything else (Float64, counts, stop
+    reasons, scalars) as Float64.  Each array gets an equal share of DUMP_BYTES; of a larger one only the entries at flat (C
+    order) positions drawn from Philox(key = crc32(name)) are kept, in ascending order - the same positions in every run."""
+    os.makedirs(path, exist_ok=True)
+    share = DUMP_BYTES // len(arrays)
+    for name, a in arrays.items():
+        a = np.asarray(a)
+        dt = np.dtype(np.float32 if a.dtype == np.float32 else np.float64)
+        if a.size * dt.itemsize > share:
+            rng = np.random.Generator(np.random.Philox(key=zlib.crc32(name.encode())))
+            a = a[np.unravel_index(np.sort(rng.choice(a.size, share // dt.itemsize, replace=False)), a.shape)]
+        np.save(os.path.join(path, name + ".npy"), np.ascontiguousarray(a, dtype=dt))
 
 
 def measured_peaks():
@@ -260,7 +284,7 @@ def fixed_budget_single(ctx, nb, synth, torch, cfg, args, iters, flush, k=None, 
     ctx.set_X(X)
     params = nb.default_params(maxiter=iters, engine=engine)
 
-    def device_step(profile):
+    def device_step(profile, factors=False):
         b = ctx.batch(k, R)
         b.init_random(SEED0)  # the same Philox streams as the pinned host factors, generated in HBM
         if flush is not None:
@@ -273,10 +297,11 @@ def fixed_budget_single(ctx, nb, synth, torch, cfg, args, iters, flush, k=None, 
         ms = ctx.last_solve_ms
         pm, pl = ctx.profile_get() if profile else (0.0, 0)
         ctx.profile(False)
-        tot = int(b.get(factors=False)["iters"].sum())
+        out = b.get(factors=factors)
+        tot = int(out["iters"].sum())
         nl = ctx.launches - l0
         b.close()
-        return ms, tot, nl, pm, pl
+        return ms, tot, nl, pm, pl, out
 
     # the clock sampler starts BEFORE the warm-up steps: nvidia-smi's start-up (NVML initialisation takes driver locks) stalled
     # the launches of the first timed step in one of two runs (301 ms instead of 224 ms, profiles/r02_bench_n1_second_outlier.json);
@@ -289,8 +314,9 @@ def fixed_budget_single(ctx, nb, synth, torch, cfg, args, iters, flush, k=None, 
     tot_ms = tot_it = launches = pass_l = 0
     pass_ms = 0.0
     step_ms = []
-    for _ in range(args.steps):
-        ms, tot, nl, pm, pl = device_step(True)
+    for s in range(args.steps):
+        # the factors of the last step come back only for --dump-outputs, after the solve's events have been read
+        ms, tot, nl, pm, pl, out = device_step(True, factors=bool(args.dump_outputs) and s == args.steps - 1)
         step_ms.append(ms)
         tot_ms += ms
         tot_it += tot
@@ -317,31 +343,36 @@ def fixed_budget_single(ctx, nb, synth, torch, cfg, args, iters, flush, k=None, 
                                                 C.byref(params), Wb.ctypes.data_as(C.c_void_p), Hb.ctypes.data_as(C.c_void_p),
                                                 C.byref(phi), C.byref(rob), C.byref(aic), C.byref(tot)), ctx._h)
         torch.cuda.synchronize()
-        return time.perf_counter() - t0, int(tot.value), rob.value
+        return time.perf_counter() - t0, int(tot.value), rob.value, phi.value, aic.value
 
     for _ in range(min(args.warmup, 1)):
         e2e_step()
     e2e_t = e2e_it = 0
     rob = None
     for _ in range(args.steps):
-        dts, t, rob = e2e_step()
+        dts, t, rob, phi, aic = e2e_step()
         e2e_t += dts
         e2e_it += t
+    if args.dump_outputs:  # what each arm's caller received in its last step: the batch of nmfk_solve, the best restart of nmfk_execute_run
+        outputs = {name: out[name] for name in BATCH_FIELDS}
+        outputs.update(e2e_W=Wb.T, e2e_H=Hb.T, e2e_fit=phi, e2e_robustness=rob, e2e_aic=aic)
+        dump_outputs(args.dump_outputs, outputs)
     return dict(value=tot_it / (tot_ms * 1e-3), ms_per_step=tot_ms / args.steps, step_ms=step_ms, iters_per_step=tot_it / args.steps,
                 launches=launches, pass_ms=pass_ms, pass_launches=pass_l, flops_per_pass=4.0 * n * m * k * R, clocks=clocks,
                 e2e_value=e2e_it / e2e_t, e2e_ms_per_step=e2e_t / args.steps * 1e3, h2d=h2d, d2h=d2h, robustness=rob,
                 n=n, m=m, k=k, R=R)
 
 
-def bench_c2(ctx, nb, synth, torch, args, flush, steps, warmup):
-    """C2 on one GPU: execute(X, 2:10, 100) with the reference stop rule (the resident DMMA engine)."""
+def bench_c2(ctx, nb, synth, torch, args, flush, steps, warmup, dump=None):
+    """C2 on one GPU: execute(X, 2:10, 100) with the reference stop rule (the resident DMMA engine).  dump: directory for what
+    the last timed step and the timed execute call returned (--dump-outputs)."""
     n, m, k0, dt, ks, R = CONFIGS["C2"]
     X = synth.mixture(n, m, k0, seed=SEED_X)
     ctx.set_X(X)
     params = nb.default_params()
     peak = max(ctx.measure_peak(1) for _ in range(2))
 
-    def step():
+    def step(factors=False):
         bs = [ctx.batch(k, R) for k in ks]
         for b in bs:
             b.init_random(SEED0)
@@ -349,22 +380,29 @@ def bench_c2(ctx, nb, synth, torch, args, flush, steps, warmup):
         torch.cuda.synchronize()
         ctx.solve(bs, params)
         ms = ctx.last_solve_ms
-        its = {b.k: int(b.get(factors=False)["iters"].sum()) for b in bs}
+        outs = {b.k: b.get(factors=factors) for b in bs}
+        its = {k: int(o["iters"].sum()) for k, o in outs.items()}
         for b in bs:
             b.close()
-        return ms, its
+        return ms, its, outs
 
     for _ in range(warmup):
         step()
     tot_ms, tot_it, flops = 0.0, 0, 0.0
-    for _ in range(steps):
-        ms, its = step()
+    for s in range(steps):
+        ms, its, outs = step(factors=bool(dump) and s == steps - 1)
         tot_ms += ms
         tot_it += sum(its.values())
         flops += sum(8.0 * n * m * k * v for k, v in its.items())
     t0 = time.perf_counter()
     W, H, fit, rob, aic, kopt = nb.execute(X, ks, R, seed=SEED0, ctx=ctx)
     e2e = time.perf_counter() - t0
+    if dump:
+        outputs = {"k%d_%s" % (k, name): o[name] for k, o in outs.items() for name in BATCH_FIELDS}
+        for k in ks:
+            outputs.update({"e2e_k%d_W" % k: W[k], "e2e_k%d_H" % k: H[k]})
+        outputs.update(e2e_fit=fit, e2e_robustness=rob, e2e_aic=aic, e2e_kopt=-1 if kopt is None else kopt)
+        dump_outputs(dump, outputs)
     tf = flops / (tot_ms * 1e-3) / 1e12
     return {"workload": WORKLOADS["C2"], "value": tot_it / (tot_ms * 1e-3), "unit": UNIT, "ms_per_step": tot_ms / steps,
             "restart_iterations_per_step": tot_it / steps, "kopt": kopt, "e2e_s_execute": e2e,
@@ -392,7 +430,13 @@ def main():
     ap.add_argument("--iters", type=int, default=0, help="iterations per step of the fixed-budget configurations")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-also", action="store_true", help="skip the secondary measurements (C2, C4 on one GPU)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the timed path returned in its last timed step as DIR/<name>.npy (less than 64 MB in all)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the outputs of the GPU path (--impl ours)")
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
@@ -575,6 +619,10 @@ def main():
         launches = ctx.launches - l0
         wall_max, solve_max, pm_max = reduce_max([wall, solve, pm])
         launches_all, = reduce_sum([float(launches)])
+        if rank == 0 and args.dump_outputs:  # the results of the last nmfk_sweep, the same on every rank
+            outputs = {"k%d_%s" % (k, name): out[name][k] for k in ks for name in ("W", "H")}
+            outputs.update(fit=out["fit"], robustness=out["robustness"], aic=out["aic"], kopt=-1 if out["kopt"] is None else out["kopt"])
+            dump_outputs(args.dump_outputs, outputs)
         # the strong-scaling anchor of THIS run: rank 0 alone repeats one step with all 256 restarts of every k on its GPU (a
         # second context without the communicator) while the other ranks wait; outside the timed region
         n1 = None
@@ -630,7 +678,7 @@ def main():
         del Xloc
         params = nb.default_params(maxiter=iters, engine=2)
 
-        def step(profile):
+        def step(profile, factors=False):
             barrier()
             t0 = time.perf_counter()
             ctx.set_X(Xpin.numpy().T)
@@ -644,8 +692,10 @@ def main():
             dts = time.perf_counter() - t0
             pm, pl = ctx.profile_get() if profile else (0.0, 0)
             ctx.profile(False)
+            if factors:  # after the timed region: this rank's rows of W and the replicated H as well
+                st = b.get()
             b.close()
-            return dts, ctx.last_solve_ms, int(st["iters"].sum()), pm, pl
+            return dts, ctx.last_solve_ms, int(st["iters"].sum()), pm, pl, st
 
         sampler = ClockSampler(local_rank)
         sampler.start()
@@ -656,9 +706,9 @@ def main():
         l0 = ctx.launches
         wall = solve = pm = 0.0
         its = pl = 0
-        for _ in range(args.steps):
+        for s in range(args.steps):
             flush.fill_(1)
-            d, s_ms, t, a, b_ = step(True)
+            d, s_ms, t, a, b_, st = step(True, factors=rank == 0 and bool(args.dump_outputs) and s == args.steps - 1)
             wall += d
             solve += s_ms
             its += t
@@ -669,6 +719,8 @@ def main():
         launches = ctx.launches - l0
         wall_max, solve_max, pm_max = reduce_max([wall, solve, pm])
         launches_all, = reduce_sum([float(launches)])
+        if rank == 0 and args.dump_outputs:  # rank 0's results: W holds rows [0, r1) of the global W, the rest is replicated
+            dump_outputs(args.dump_outputs, {name: st[name] for name in BATCH_FIELDS})
         if rank == 0:
             nloc = r1 - r0
             achieved = 4.0 * nloc * m * k * R * pl / (pm_max * 1e-3) / 1e12 if pm_max > 0 else float("nan")
@@ -694,7 +746,7 @@ def main():
     elif cfg == "C2":
         if world != 1:
             raise SystemExit("bench.py: --config C2 runs on one GPU")
-        r = bench_c2(ctx, nb, synth, torch, args, flush, args.steps, args.warmup)
+        r = bench_c2(ctx, nb, synth, torch, args, flush, args.steps, args.warmup, dump=args.dump_outputs)
         line = {"metric": METRIC, "value": r["value"], "unit": UNIT, "n_gpus": 1, "steps": args.steps, "warmup": args.warmup,
                 "ms_per_step": r["ms_per_step"], "higher_is_better": True, "scaling": "weak", "vs_baseline": None, "dtype": "f64",
                 "data": "synthetic", "config": {"workload": WORKLOADS["C2"], "kopt": r["kopt"], "same_config": True,
