@@ -899,7 +899,7 @@ int32_t nmfk_solve(nmfk_ctx* c, nmfk_batch* const* batches, int32_t nb, const nm
         }
         if ((p->engine == NMFK_ENGINE_RESIDENT || p->engine == NMFK_ENGINE_RESIDENT_SCALAR) && !resident)
             return fail(c, NMFK_E_UNSUPPORTED, "resident engine: factors do not fit in shared memory (or k > 32)");
-        if (!resident && !tiled_supported(a.k)) return fail(c, NMFK_E_UNSUPPORTED, "tiled engine: k > 32 is not supported");
+        if (!resident && !tiled_supported(a.k)) return fail(c, NMFK_E_UNSUPPORTED, "tiled engine: k > 64 is not supported");
         mode[q] = resident ? (fits_dmma ? 1 : 2) : 3;
     }
     for (int lim = std::min(kResidentChunk, user_limit);; lim = std::min(lim + kResidentChunk, user_limit)) {

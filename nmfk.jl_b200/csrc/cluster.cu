@@ -527,6 +527,8 @@ cudaError_t launch_point_silhouettes(double* V, int len, int ld, int N, int k, c
     if ((e = pairwise_cosine(V, len, ld, N, vnorm, Dm, s)) != cudaSuccess) return e;
     const int NT = 128;
     const size_t smem = (size_t)k * NT * sizeof(double) + (size_t)k * sizeof(int);
+    if (smem > 48 * 1024 && (e = cudaFuncSetAttribute(silhouette_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem)) != cudaSuccess)
+        return e;
     silhouette_kernel<<<(N + NT - 1) / NT, NT, smem, s>>>(Dm, N, k, labels, sil);
     return cudaGetLastError();
 }
@@ -588,6 +590,9 @@ cudaError_t launch_cluster(const ClusterArgs& a, int dtype, cudaStream_t s) {
         if ((e = pairwise_cosine(a.V, a.len, ld, N, a.vnorm, a.Dm, s)) != cudaSuccess) return e;
         const int NT = 128;
         const size_t smem = (size_t)a.k * NT * sizeof(double) + (size_t)a.k * sizeof(int);
+        if (smem > 48 * 1024 &&  // k >= 48
+            (e = cudaFuncSetAttribute(silhouette_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem)) != cudaSuccess)
+            return e;
         silhouette_kernel<<<(N + NT - 1) / NT, NT, smem, s>>>(a.Dm, N, a.k, a.labels, a.sil);
         if ((e = cudaGetLastError()) != cudaSuccess) return e;
         cluster_mean_kernel<<<1, 64, 0, s>>>(a.sil, a.labels, N, a.k, a.clustersil);

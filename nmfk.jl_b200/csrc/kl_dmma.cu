@@ -19,7 +19,7 @@ struct DmmaPlan {
 
 // template K instantiated for a requested k: exact up to 12, then multiples of 4
 int dmma_template_k(int k) {
-    if (k < 1 || k > kMaxK) return -1;
+    if (k < 1 || k > kResidentMaxK) return -1;
     if (k <= 12) return k;
     return (k + 3) / 4 * 4;
 }

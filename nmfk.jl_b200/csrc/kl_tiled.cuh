@@ -155,7 +155,7 @@ __global__ void __launch_bounds__(kTiledThreads, (K <= 12 ? 2 : 1)) tiled_pass_k
     cp_async_wait<0>();
     if (!valid) return;
     if (a.partial == nullptr) {
-        const TC* den = static_cast<const TC*>(a.den) + (long long)r * 32;
+        const TC* den = static_cast<const TC*>(a.den) + (long long)r * kTiledMaxK;
 #pragma unroll
         for (int c = 0; c < K; ++c)
             if (c < k) U[(long long)o * a.su_o + (long long)c * a.su_a] = div_cold<TC>(u[c] * acc[c], den[c]);
@@ -176,7 +176,7 @@ __global__ void tiled_combine_kernel(const TiledPassArgs a, TC* __restrict__ red
     const int o = blockIdx.x * blockDim.x + threadIdx.x;
     if (o >= a.nown) return;
     TC* U = static_cast<TC*>(a.U) + (long long)r * a.u_rstride;
-    const TC* den = static_cast<const TC*>(a.den) + (long long)r * 32;
+    const TC* den = static_cast<const TC*>(a.den) + (long long)r * kTiledMaxK;
     TC acc[K];
 #pragma unroll
     for (int c = 0; c < K; ++c) acc[c] = (TC)0;
@@ -207,7 +207,7 @@ __global__ void tiled_apply_kernel(const TiledPassArgs a, const TC* __restrict__
     const int o = blockIdx.x * blockDim.x + threadIdx.x;
     if (o >= a.nown) return;
     TC* U = static_cast<TC*>(a.U) + (long long)r * a.u_rstride;
-    const TC* den = static_cast<const TC*>(a.den) + (long long)r * 32;
+    const TC* den = static_cast<const TC*>(a.den) + (long long)r * kTiledMaxK;
     const TC* src = red + ((long long)r * a.nown + o) * K;
 #pragma unroll
     for (int c = 0; c < K; ++c)
@@ -251,7 +251,7 @@ __global__ void __launch_bounds__(256) tiled_sums_kernel(const void* Vv, long lo
     for (; t < nred; t += NT) s0 += (double)V[(long long)t * sv_t];
     double s = (s0 + s1) + (s2 + s3);
     s = block_sum(s, red);
-    if (threadIdx.x == 0) static_cast<TC*>(denv)[(long long)r * 32 + c] = (TC)s;
+    if (threadIdx.x == 0) static_cast<TC*>(denv)[(long long)r * kTiledMaxK + c] = (TC)s;
 }
 
 // sum over non-NaN entries of ((x - W_r H_r) w)^2 and (x - W_r H_r)^2 for 128 rows x all columns;
@@ -307,6 +307,15 @@ __global__ void __launch_bounds__(128) tiled_objective_kernel(const TX* __restri
         partials[((long long)r * gridDim.x + b) * 2] = a0;
         partials[((long long)r * gridDim.x + b) * 2 + 1] = a1;
     }
+}
+
+// the rows of W a block of tiled_objective_kernel keeps in shared memory: with the static sums above 48 KB (Float64, k >= 48)
+// only with the attribute
+template <typename TX, typename TC>
+cudaError_t tiled_objective_smem(int k) {
+    const size_t smem = (size_t)k * 128 * sizeof(TC);
+    if (smem + sizeof(double) * 2 * 4 <= 48 * 1024) return cudaSuccess;
+    return cudaFuncSetAttribute(tiled_objective_kernel<TX, TC>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
 }
 
 // X[inan] = (W*H)[inan] (:72) for every running restart
@@ -473,7 +482,7 @@ __global__ void __launch_bounds__(256) tiled_scaleW_kernel(TC* __restrict__ Wst,
     const int r = blockIdx.y;
     if (!wflag[r]) return;
     TC* W = Wst + (long long)r * n * k;
-    const double* t = tot + (long long)r * 32;
+    const double* t = tot + (long long)r * kTiledMaxK;
     const long long nk = n * k;
     for (long long e = (long long)blockIdx.x * blockDim.x + threadIdx.x; e < nk; e += (long long)gridDim.x * blockDim.x)
         W[e] = W[e] * (TC)t[e / n];
@@ -484,7 +493,7 @@ __global__ void __launch_bounds__(256) tiled_finish_kernel(void* Wv, void* Hv, U
                                                            int n, int m, int k, int nblk, int normalize, double* tot_out = nullptr,
                                                            int* wflag = nullptr) {
     __shared__ double red[40];
-    __shared__ double tot[32];
+    __shared__ double tot[kTiledMaxK];
     const int r = blockIdx.x, tid = threadIdx.x, NT = blockDim.x;
     UnitState* st = stv + r;
     if (st->stop == 0 || st->done != 0) return;
@@ -508,7 +517,7 @@ __global__ void __launch_bounds__(256) tiled_finish_kernel(void* Wv, void* Hv, U
         }
         __syncthreads();
         if (wflag != nullptr) {  // W is scaled by tiled_scaleW_kernel over the whole GPU
-            for (int c = tid; c < k; c += NT) tot_out[(long long)r * 32 + c] = tot[c];
+            for (int c = tid; c < k; c += NT) tot_out[(long long)r * kTiledMaxK + c] = tot[c];
             if (tid == 0) wflag[r] = 1;
         } else {
             for (long long e = tid; e < (long long)n * k; e += NT) W[e] = W[e] * (TC)tot[e / n];
@@ -598,17 +607,44 @@ cudaError_t launch_tiled_apply_k(const TiledPassArgs& a, void* red, cudaStream_t
 // ------------------------------------------------------------------------------------------
 namespace nmfk {
 
+// template K of the tiled engine's kernels (tiled_template_k): the resident set up to 32, then 40 / 48 / 56 / 64.  Kept
+// apart from NMFK_DISPATCH_K so that no resident kernel is instantiated above 32.
+#define NMFK_DISPATCH_TILED_K(FN, TX, TC, KT, ...)                \
+    switch (KT) {                                                 \
+        case 1: return FN<TX, TC, 1>(__VA_ARGS__);                \
+        case 2: return FN<TX, TC, 2>(__VA_ARGS__);                \
+        case 3: return FN<TX, TC, 3>(__VA_ARGS__);                \
+        case 4: return FN<TX, TC, 4>(__VA_ARGS__);                \
+        case 5: return FN<TX, TC, 5>(__VA_ARGS__);                \
+        case 6: return FN<TX, TC, 6>(__VA_ARGS__);                \
+        case 7: return FN<TX, TC, 7>(__VA_ARGS__);                \
+        case 8: return FN<TX, TC, 8>(__VA_ARGS__);                \
+        case 9: return FN<TX, TC, 9>(__VA_ARGS__);                \
+        case 10: return FN<TX, TC, 10>(__VA_ARGS__);              \
+        case 11: return FN<TX, TC, 11>(__VA_ARGS__);              \
+        case 12: return FN<TX, TC, 12>(__VA_ARGS__);              \
+        case 16: return FN<TX, TC, 16>(__VA_ARGS__);              \
+        case 20: return FN<TX, TC, 20>(__VA_ARGS__);              \
+        case 24: return FN<TX, TC, 24>(__VA_ARGS__);              \
+        case 32: return FN<TX, TC, 32>(__VA_ARGS__);              \
+        case 40: return FN<TX, TC, 40>(__VA_ARGS__);              \
+        case 48: return FN<TX, TC, 48>(__VA_ARGS__);              \
+        case 56: return FN<TX, TC, 56>(__VA_ARGS__);              \
+        case 64: return FN<TX, TC, 64>(__VA_ARGS__);              \
+        default: return cudaErrorInvalidValue;                    \
+    }
+
 template <typename TX, typename TC>
 cudaError_t dispatch_tiled_combine(const TiledPassArgs& a, void* red, cudaStream_t s) {
-    const int kt = resident_template_k(a.k);
-    NMFK_DISPATCH_K(launch_tiled_combine_k, TX, TC, kt, a, red, s)
+    const int kt = tiled_template_k(a.k);
+    NMFK_DISPATCH_TILED_K(launch_tiled_combine_k, TX, TC, kt, a, red, s)
 }
 // use_tc: Float32 without NaN -> the tcgen05 kernel of kl_tiled_tc.cu (a.nblocks counts 128-index tiles)
 // use_td: Float64 without NaN, k >= 4 -> the DMMA kernel of kl_tiled_dmma.cu (a.nblocks counts 128-index blocks, a.D is
 // the step-contiguous copy of the data)
 template <typename TX, typename TC>
 cudaError_t dispatch_tiled_pass(const TiledPassArgs& a, void* red, cudaStream_t s, bool use_tc, int* errflag, bool use_td = false) {
-    const int kt = resident_template_k(a.k);
+    const int kt = tiled_template_k(a.k);
     if (use_tc) {
         cudaError_t e = launch_tc_pass(a, errflag, s);
         if (e != cudaSuccess || a.partial == nullptr) return e;
@@ -619,7 +655,7 @@ cudaError_t dispatch_tiled_pass(const TiledPassArgs& a, void* red, cudaStream_t 
         if (e != cudaSuccess || a.partial == nullptr) return e;
         return dispatch_tiled_combine<TX, TC>(a, red, s);
     }
-    NMFK_DISPATCH_K(launch_tiled_pass_k, TX, TC, kt, a, red, s)
+    NMFK_DISPATCH_TILED_K(launch_tiled_pass_k, TX, TC, kt, a, red, s)
 }
 // the same, bracketed by the profile events (one "launch" = the pass kernel, plus the small slice-combine kernel when the
 // reduction range is sliced)
@@ -633,8 +669,8 @@ cudaError_t timed_tiled_pass(const TiledPassArgs& a, void* red, cudaStream_t s, 
 }
 template <typename TX, typename TC>
 cudaError_t dispatch_tiled_apply(const TiledPassArgs& a, void* red, cudaStream_t s) {
-    const int kt = resident_template_k(a.k);
-    NMFK_DISPATCH_K(launch_tiled_apply_k, TX, TC, kt, a, red, s)
+    const int kt = tiled_template_k(a.k);
+    NMFK_DISPATCH_TILED_K(launch_tiled_apply_k, TX, TC, kt, a, red, s)
 }
 
 // NMFK_TILED_TIMING=1: device time of every phase of the tiled engine's iteration (CUDA events between the launches, read at
@@ -694,7 +730,7 @@ struct PhaseTimer {
 template <typename TX, typename TC>
 cudaError_t solve_tiled_t(const SolveArgs& a, cudaStream_t s, int64_t* launches) {
     const int n = a.n, m = a.m, k = a.k, R = a.R;
-    const int kt = resident_template_k(k);
+    const int kt = tiled_template_k(k);
     if (kt < 0) return cudaErrorInvalidValue;
     cudaError_t err = cudaSuccess;
     int sms = 148;
@@ -756,7 +792,7 @@ cudaError_t solve_tiled_t(const SolveArgs& a, cudaStream_t s, int64_t* launches)
     double host_setup_ms = 0.0;
     const int it_begin_report = 0;
     (void)it_begin_report;
-    TC* den = nullptr;  // R x 32, followed by red (R x m x kt) when sharded
+    TC* den = nullptr;  // R x kTiledMaxK, followed by red (R x m x kt) when sharded
     TC* red = nullptr;
     double* obj2 = nullptr;
     TC* partial = nullptr;
@@ -808,13 +844,13 @@ cudaError_t solve_tiled_t(const SolveArgs& a, cudaStream_t s, int64_t* launches)
     };
   // column sums of W would need another exchange
 
-    NMFK_TRY(scratch_alloc(&den, ((size_t)R * 32 + redsz) * sizeof(TC), s));
-    if (sharded) red = den + (size_t)R * 32;
+    NMFK_TRY(scratch_alloc(&den, ((size_t)R * kTiledMaxK + redsz) * sizeof(TC), s));
+    if (sharded) red = den + (size_t)R * kTiledMaxK;
     NMFK_TRY(scratch_alloc(&obj2, (size_t)R * 2 * sizeof(double), s));
     if (psz) NMFK_TRY(scratch_alloc(&partial, psz * sizeof(TC), s));
     NMFK_TRY(scratch_alloc(&objp, (size_t)R * nblkObj * 2 * sizeof(double), s));
     NMFK_TRY(scratch_alloc(&d_active, sizeof(int), s));
-    NMFK_TRY(scratch_alloc(&fin_tot, (size_t)R * 32 * sizeof(double), s));
+    NMFK_TRY(scratch_alloc(&fin_tot, (size_t)R * kTiledMaxK * sizeof(double), s));
     NMFK_TRY(scratch_alloc(&fin_flag, (size_t)R * sizeof(int), s));
     h_active = pinned_flags();
     if (h_active == nullptr) NMFK_TRY(cudaErrorMemoryAllocation);
@@ -929,7 +965,7 @@ cudaError_t solve_tiled_t(const SolveArgs& a, cudaStream_t s, int64_t* launches)
                 }
                 if (sharded) {
                     // colsum(W) and W' * (X ./ (W*H)) over this rank's rows -> sums over all rows, then the update
-                    NMFK_TRY(sh->allreduce(sh->comm, den, (size_t)R * 32 + redsz, sizeof(TC) == 8 ? 1 : 0, s));
+                    NMFK_TRY(sh->allreduce(sh->comm, den, (size_t)R * kTiledMaxK + redsz, sizeof(TC) == 8 ? 1 : 0, s));
                     pt.mark(s, 2);
                     NMFK_TRY((dispatch_tiled_apply<TX, TC>(ph, red, s)));
                     pt.mark(s, 3);
@@ -958,6 +994,7 @@ cudaError_t solve_tiled_t(const SolveArgs& a, cudaStream_t s, int64_t* launches)
                     NMFK_TRY(launch_tiled_dmma_objective(obj_args(0, 0), s));
                 } else {
                     dim3 g(nblkObj, R);
+                    NMFK_TRY((tiled_objective_smem<TX, TC>(k)));
                     tiled_objective_kernel<TX, TC><<<g, 128, (size_t)k * 128 * sizeof(TC), s>>>(
                         (const TX*)a.X, n, m, k, (const TC*)a.W, (const TC*)a.H, a.st, (TC)a.lambda, 0, 1, a.weight, a.wref, objp);
                 }
@@ -1018,6 +1055,7 @@ cudaError_t solve_tiled_t(const SolveArgs& a, cudaStream_t s, int64_t* launches)
             NMFK_TRY(launch_tiled_dmma_objective(obj_args(1, 1), s));
         } else {
             dim3 g(nblkObj, R);
+            NMFK_TRY((tiled_objective_smem<TX, TC>(k)));
             tiled_objective_kernel<TX, TC><<<g, 128, (size_t)k * 128 * sizeof(TC), s>>>(
                 (const TX*)a.X, n, m, k, (const TC*)a.W, (const TC*)a.H, a.st, (TC)a.lambda, 1, 0, a.weight, a.wref, objp);
         }

@@ -8,7 +8,7 @@ struct TiledPassArgs {
     const void* D;      // data in "own-contiguous" layout: element (o,t) at D[o + t*nown]
     void* U;            // own factor stack
     const void* V;      // broadcast factor stack
-    const void* den;    // R x 32 : sum_t V[t,a]
+    const void* den;    // R x kTiledMaxK : sum_t V[t,a]
     void* partial;      // slices x R x nown x K partial numerators (S > 1) or nullptr
     const UnitState* st;
     const void* ximp;   // R x n x m (X layout) or nullptr
@@ -49,7 +49,7 @@ cudaError_t launch_tc_objective(const TiledPassArgs& a, int* d_errflag, cudaStre
 
 // Float64 half-update on the FP64 tensor pipe (kl_tiled_dmma.cu): DMMA fragment formulation of the resident engine with
 // the other factor streamed through shared memory.  a.D = STEP-contiguous data (H-update: X, W-update: X^T),
-// nblocks = ceil(nown / tiled_dmma_own()), 4 <= k <= 32, no NaN.
+// nblocks = ceil(nown / tiled_dmma_own()), 4 <= k <= 64, no NaN.
 int tiled_dmma_own();
 int tiled_dmma_chunk();
 cudaError_t launch_tiled_dmma_pass(const TiledPassArgs& a, cudaStream_t s);

@@ -1,5 +1,5 @@
 // Float64 half-update of the tiled KL engine on the FP64 tensor pipe (DMMA m8n8k4), for factors that do not fit
-// in shared memory (BASELINE config C4: 100000 x 2000 Float64, k = 2:32, nNMF = 256).
+// in shared memory (BASELINE config C4: 100000 x 2000 Float64, k = 2:32, nNMF = 256; the tiled engine takes k up to 64).
 //
 // Replaces, for Float64 data without NaN, the loop body of NMFk.NMFmultiplicative
 // (/root/reference/src/NMFkMultiplicative.jl:67,70) exactly like tiled_pass_kernel (kl_tiled.cuh):
@@ -213,7 +213,7 @@ __global__ void __launch_bounds__(TD_THREADS, 1) tiled_dmma_pass_kernel(const Ti
     R.finish();
     if (!rvalid) return;
     if (a.partial == nullptr) {
-        const double* den = static_cast<const double*>(a.den) + (long long)r * 32;
+        const double* den = static_cast<const double*>(a.den) + (long long)r * kTiledMaxK;
 #pragma unroll
         for (int v = 0; v < NV; ++v) {
             const int c = DmmaRegs<K>::column(v, q);
@@ -259,6 +259,10 @@ cudaError_t dispatch_td(const TiledPassArgs& a, cudaStream_t s) {
         case 20: return launch_td<20, OBJ>(a, s);
         case 24: return launch_td<24, OBJ>(a, s);
         case 32: return launch_td<32, OBJ>(a, s);
+        case 40: return launch_td<40, OBJ>(a, s);
+        case 48: return launch_td<48, OBJ>(a, s);
+        case 56: return launch_td<56, OBJ>(a, s);
+        case 64: return launch_td<64, OBJ>(a, s);
         default: return cudaErrorInvalidValue;
     }
 }
@@ -268,8 +272,8 @@ cudaError_t dispatch_td(const TiledPassArgs& a, cudaStream_t s) {
 int tiled_dmma_own() { return TD_OWN; }
 int tiled_dmma_chunk() { return TD_TCH; }
 
-// a.k in 4..32 (smaller k are all-DFMA in the resident formulation and stay on the scalar pass); K = the template K of
-// the combine kernel (resident_template_k), a.nblocks = ceil(nown / 128), a.D step-contiguous
+// a.k in 4..64 (smaller k are all-DFMA in the resident formulation and stay on the scalar pass); K = the template K of
+// the combine kernel (tiled_template_k), a.nblocks = ceil(nown / 128), a.D step-contiguous
 cudaError_t launch_tiled_dmma_pass(const TiledPassArgs& a, cudaStream_t s) { return dispatch_td<false>(a, s); }
 // objective sums: a = the W-update arguments (D = X^T step-contiguous, U = W, V = H), S = 1
 cudaError_t launch_tiled_dmma_objective(const TiledPassArgs& a, cudaStream_t s) { return dispatch_td<true>(a, s); }

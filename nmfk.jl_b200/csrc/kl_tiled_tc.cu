@@ -25,6 +25,10 @@
 // Tensor-memory map (512 columns): [0,256) two P/Q buffers (64 P->Qhi + 64 Qlo), then two per-unit numerator
 // buffers (NST*N2 columns each; k <= 16 stacks Qhi*[Vhi;Vlo] into one N = 32 instruction), then U hi | U lo
 // (K8 each) per restart of the group.
+// 32 < k <= 64 (N2 = 64): 256 + 128 + 2 K8 columns leave room for ONE restart per CTA (RB = 1; X tiles are no longer shared
+// between restarts, they come from L2 for the other restarts' CTAs); the two quotient groups then alternate chunks of the
+// same restart and add their numerators at the end.  Shared memory: 2 X stages + 2 V images (64 KB each at K8 = 64) + 2 raw
+// chunks = 224 KB.
 #include <algorithm>
 
 #include "kl_tiled_args.h"
@@ -43,9 +47,10 @@ constexpr int TC_M = 128;
 template <int K8, int N2>
 struct TcCfg {
     static constexpr int TS = 64;                                     // steps per chunk
-    static constexpr int NXS = 3;                                     // X tile stages
-    static constexpr int NRAW = 4;                                    // raw V chunk buffers
-    static constexpr int NVB = K8 <= 16 ? 4 : 3;                      // V image buffers (shared memory budget for k > 16)
+    // X tile stages, raw V chunk buffers, V image buffers: fewer as the V images grow (shared memory budget for k > 16 / 32)
+    static constexpr int NXS = K8 <= 32 ? 3 : 2;
+    static constexpr int NRAW = K8 <= 32 ? 4 : 2;
+    static constexpr int NVB = K8 <= 16 ? 4 : (K8 <= 32 ? 3 : 2);
     static constexpr int RPAD = K8 > 24 ? 0 : 4;                      // raw V chunk padding (shared memory budget at K8 = 32)
     static constexpr int QW = TS / 4;                                 // quotient warps: lane quarter = warp % 4, 16 columns each
     static constexpr int SW = 4;                                      // V stager warps
@@ -147,11 +152,12 @@ __global__ void __launch_bounds__((TcCfg<K8, N2>::THREADS), 1) tc_pass_kernel(co
         s_act[RB] = nact;
         // pass mode: the two quotient groups alternate units, so a chunk holds an EVEN number of units; an odd group of
         // restarts (ragged last group, frozen restarts) gets a shadow unit that recomputes its first restart and is dropped
-        if (!OBJ && (nact & 1)) s_act[nact] = s_act[0];
+        // (one restart per CTA, k > 32: the groups alternate chunks instead)
+        if (!OBJ && RB > 1 && (nact & 1)) s_act[nact] = s_act[0];
     }
     __syncthreads();
     const int nreal = s_act[RB];
-    const int nact = OBJ ? nreal : nreal + (nreal & 1);
+    const int nact = (OBJ || RB == 1) ? nreal : nreal + (nreal & 1);
     if (nreal == 0 || nchunks <= 0) return;
     const int total = nchunks * nact;
 
@@ -399,7 +405,10 @@ __global__ void __launch_bounds__((TcCfg<K8, N2>::THREADS), 1) tc_pass_kernel(co
         // slower); the a_full wait that precedes it has normally completed long before.
         // The 16 numerator values of a thread (NST = 2: 8 columns of Qhi*Vhi+Qlo*Vhi and the same 8 of Qhi*Vlo; NST = 1:
         // 16 columns) are fetched in two parts of 8, one per 16-column round of the division, to keep registers down.
-        static_assert(NC2 * C::NST == 16, "numerator values per quotient thread");
+        // N2 = 64 (k > 32, one restart slot): 32 numerator values, added before the division in four loads of 8 (DRAIN32) - with
+        // 32 accumulators, a prefetch next to the 2 x 16 quotient registers spilled part of them to local memory.
+        constexpr bool DRAIN32 = NC2 == 32;
+        static_assert(NC2 * C::NST == 16 || (DRAIN32 && SL == 1), "numerator values per quotient thread");
         uint32_t v[8];
         const uint32_t acol = lane_base + C::ABASE + (uint32_t)grp * C::ACOLS + hh * NC2;
         auto drain_load = [&](int part) { tc::tmem_ld8(acol + part * (C::NST == 2 ? N2 : 8), v); };
@@ -419,14 +428,27 @@ __global__ void __launch_bounds__((TcCfg<K8, N2>::THREADS), 1) tc_pass_kernel(co
                     }
                 }
         };
+        auto drain32 = [&]() {
+#pragma unroll
+            for (int q = 0; q < NC2 / 8; ++q) {
+                tc::tmem_ld8(acol + q * 8, v);
+                tc::tmem_wait_ld();
+#pragma unroll
+                for (int c = 0; c < 8; ++c) acc[0][q * 8 + c] += __uint_as_float(v[c]);
+            }
+        };
+        // One restart per CTA (RB = 1, k > 32): the groups take the even / odd CHUNKS, both accumulate the same restart and
+        // their sums are added at the end.
         int prev_slot = -1;  // restart slot index (b / 2) of this group's previous unit, -1: none yet
+        int ulast = -1;      // this group's last unit
         for (int c = 0; c < nchunks; ++c) {
             const int s = c % TC_NXS;
             const int cnt = min(TC_TS, t_end - (t_begin + c * TC_TS));
             tc::mbar_wait_h(0u, &x_full[s], (uint32_t)((c / TC_NXS) & 1), errflag, 40);
             const float* xs = Xs + (size_t)s * TC_TS * TC_M + (size_t)jh * TC_M + o_loc;
-            for (int b = grp; b < nact; b += 2) {
-                const int u = c * nact + b;  // u % 2 == grp (nact is even)
+            for (int b = RB == 1 ? 0 : grp; b < nact; b += 2) {
+                const int u = c * nact + b;  // u % 2 == grp when nact is even
+                if (RB == 1 && (u & 1) != grp) continue;
                 const int pq = u % C::NPQ;
                 const uint32_t col = lane_base + (uint32_t)pq * C::PQ + jh;
                 if (warp == TC_QW0) TC_STAMP(0, u, 0);
@@ -439,12 +461,14 @@ __global__ void __launch_bounds__((TcCfg<K8, N2>::THREADS), 1) tc_pass_kernel(co
                 if (prev_slot >= 0) tc::mbar_wait_h(0u, &a_full[grp], (uint32_t)((((u - 2) >> 1)) & 1), errflag, 44);
                 tc::tc_fence_after_sync();
                 if (warp == TC_QW0) TC_STAMP(0, u, 1);
+                if constexpr (DRAIN32)
+                    if (prev_slot >= 0) drain32();
 #pragma unroll 1
                 for (int half = 0; half < 2; ++half) {
                     uint32_t p[16], lo[16];
                     tc::tmem_ld16(col + half * 16, p);
                     tc::tmem_wait_ld();
-                    if (prev_slot >= 0) drain_load(half);
+                    if (!DRAIN32 && prev_slot >= 0) drain_load(half);
                     if (half == 0 && warp == TC_QW0) TC_STAMP(0, u, 2);
                     const float* xh = xs + half * 16 * TC_M;
                     if (cnt == TC_TS) {
@@ -474,7 +498,7 @@ __global__ void __launch_bounds__((TcCfg<K8, N2>::THREADS), 1) tc_pass_kernel(co
                             p[j] = h;
                         }
                     }
-                    if (prev_slot >= 0) {
+                    if (!DRAIN32 && prev_slot >= 0) {
                         tc::tmem_wait_ld();
                         drain_add(prev_slot, half);
                     }
@@ -488,21 +512,38 @@ __global__ void __launch_bounds__((TcCfg<K8, N2>::THREADS), 1) tc_pass_kernel(co
                 if (lane == 0) tc::mbar_arrive(&q_full[pq]);
                 if (warp == TC_QW0) TC_STAMP(0, u, 4);
                 prev_slot = b >> 1;
+                ulast = u;
             }
             __syncwarp();
             if (lane == 0) tc::mbar_arrive(&x_empty[s]);
         }
         // tail: this group's last unit waits for the commit behind its own MMA#2
-        {
-            const int ulast = (nchunks - 1) * nact + (nact - 2 + grp);
+        if (ulast >= 0) {
             tc::mbar_wait_h(0u, &a_full[grp], (uint32_t)((ulast >> 1) & 1), errflag, 43);
             tc::tc_fence_after_sync();
+            if constexpr (DRAIN32) {
+                drain32();
+            } else {
 #pragma unroll
-            for (int part = 0; part < 2; ++part) {
-                drain_load(part);
-                tc::tmem_wait_ld();
-                drain_add(prev_slot, part);
+                for (int part = 0; part < 2; ++part) {
+                    drain_load(part);
+                    tc::tmem_wait_ld();
+                    drain_add(prev_slot, part);
+                }
             }
+        }
+        if constexpr (RB == 1) {  // group 1's sums -> group 0 through the idle X stages, added in a fixed order
+            float* xch = Xs;
+            const int slot = (lq * 2 + hh) * 32 + lane;
+            __syncwarp();
+            tc::named_bar_sync(2, TC_QWARPS * 32);  // every quotient warp is past its last X tile
+            if (grp == 1)
+#pragma unroll
+                for (int c = 0; c < NC2; ++c) xch[c * 256 + slot] = acc[0][c];
+            tc::named_bar_sync(2, TC_QWARPS * 32);
+            if (grp == 0)
+#pragma unroll
+                for (int c = 0; c < NC2; ++c) acc[0][c] += xch[c * 256 + slot];
         }
         // numerators -> factor update (or the slice's partial sums): this thread's NC2 columns of this group's restarts
 #pragma unroll
@@ -512,7 +553,7 @@ __global__ void __launch_bounds__((TcCfg<K8, N2>::THREADS), 1) tc_pass_kernel(co
                 const int r = s_act[b];
                 if (a.partial == nullptr) {
                     float* U = Ug + (long long)r * a.u_rstride;
-                    const float* den = static_cast<const float*>(a.den) + (long long)r * 32;
+                    const float* den = static_cast<const float*>(a.den) + (long long)r * kTiledMaxK;
 #pragma unroll
                     for (int c = 0; c < NC2; ++c) {
                         const int col = hh * NC2 + c;
@@ -557,14 +598,16 @@ int tc_pass_group(int k) {
     if (k <= 8) return TcCfg<8, 16>::RB;
     if (k <= 16) return TcCfg<16, 16>::RB;
     if (k <= 24) return TcCfg<24, 32>::RB;
-    return TcCfg<32, 32>::RB;
+    if (k <= 32) return TcCfg<32, 32>::RB;
+    if (k <= 48) return TcCfg<48, 64>::RB;
+    return TcCfg<64, 64>::RB;
 }
 int tc_pass_ctas_per_sm(int) { return 1; }
 int tc_pass_chunk(int) { return 64; }
 
 // bulk copies need 16-byte aligned rows of 128 own indices: nown % 4 == 0
 bool tc_pass_supported(const TiledPassArgs& a) {
-    return !a.has_nan && a.k >= 1 && a.k <= 32 && (a.nown % 4) == 0 && (reinterpret_cast<uintptr_t>(a.D) % 16) == 0;
+    return !a.has_nan && a.k >= 1 && a.k <= kTiledMaxK && (a.nown % 4) == 0 && (reinterpret_cast<uintptr_t>(a.D) % 16) == 0;
 }
 
 cudaError_t launch_tc_pass(const TiledPassArgs& a, int* d_errflag, cudaStream_t s) {
@@ -572,14 +615,18 @@ cudaError_t launch_tc_pass(const TiledPassArgs& a, int* d_errflag, cudaStream_t 
     if (a.k <= 8) return launch_tc<8, 16, false>(a, d_errflag, s);
     if (a.k <= 16) return launch_tc<16, 16, false>(a, d_errflag, s);
     if (a.k <= 24) return launch_tc<24, 32, false>(a, d_errflag, s);
-    return launch_tc<32, 32, false>(a, d_errflag, s);
+    if (a.k <= 32) return launch_tc<32, 32, false>(a, d_errflag, s);
+    if (a.k <= 48) return launch_tc<48, 64, false>(a, d_errflag, s);
+    return launch_tc<64, 64, false>(a, d_errflag, s);
 }
 
 cudaError_t launch_tc_objective(const TiledPassArgs& a, int* d_errflag, cudaStream_t s) {
     if (a.k <= 8) return launch_tc<8, 16, true>(a, d_errflag, s);
     if (a.k <= 16) return launch_tc<16, 16, true>(a, d_errflag, s);
     if (a.k <= 24) return launch_tc<24, 32, true>(a, d_errflag, s);
-    return launch_tc<32, 32, true>(a, d_errflag, s);
+    if (a.k <= 32) return launch_tc<32, 32, true>(a, d_errflag, s);
+    if (a.k <= 48) return launch_tc<48, 64, true>(a, d_errflag, s);
+    return launch_tc<64, 64, true>(a, d_errflag, s);
 }
 
 }  // namespace nmfk

@@ -423,7 +423,7 @@ __global__ void __launch_bounds__((Tc2Cfg<K8>::THREADS), 1) tc2_pass_kernel(cons
                 const int r = s_act[b];
                 if (a.partial == nullptr) {
                     float* U = Ug + (long long)r * a.u_rstride;
-                    const float* den = static_cast<const float*>(a.den) + (long long)r * 32;
+                    const float* den = static_cast<const float*>(a.den) + (long long)r * kTiledMaxK;
 #pragma unroll
                     for (int c = 0; c < NC2; ++c) {
                         const int col = hh * NC2 + c;

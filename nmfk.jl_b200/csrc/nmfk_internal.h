@@ -123,7 +123,9 @@ struct SolveArgs {
 
 // threads per restart-CTA of the resident engine: 512 (<=128 registers) while u/acc fit, 256 beyond
 __host__ __device__ constexpr int resident_threads(int Ktemplate) { return Ktemplate <= 12 ? 512 : 256; }
-constexpr int kMaxK = 32;
+// largest k of the resident engines (factors in shared memory) and of the tiled engine (factors streamed)
+constexpr int kResidentMaxK = 32;
+constexpr int kTiledMaxK = 64;
 
 // template K actually instantiated for a requested k (exact up to 12, then padded)
 inline int resident_template_k(int k) {
@@ -132,6 +134,12 @@ inline int resident_template_k(int k) {
     if (k <= 20) return 20;
     if (k <= 24) return 24;
     if (k <= 32) return 32;
+    return -1;
+}
+// the same for the tiled engine: identical up to 32, then padded to a multiple of 8
+inline int tiled_template_k(int k) {
+    if (k <= kResidentMaxK) return resident_template_k(k);
+    if (k <= kTiledMaxK) return (k + 7) / 8 * 8;
     return -1;
 }
 

@@ -79,6 +79,11 @@ cudaError_t launch_residual(const void* X, int dtype, int n, int m, int k, const
     const int slices = residual_slices(n, m);
     const dim3 grid((n + kRows - 1) / kRows, slices);
     const size_t smem = (size_t)k * kRows * (dtype == 1 ? 8 : 4);
+    if (smem + sizeof(double) * 2 * (kRows / 32) > 48 * 1024) {  // the rows of W of a block, with the static sums (k >= 48 in Float64)
+        const cudaError_t e = dtype == 1 ? cudaFuncSetAttribute(residual_kernel<double>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem)
+                                         : cudaFuncSetAttribute(residual_kernel<float>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+        if (e != cudaSuccess) return e;
+    }
     if (dtype == 1)
         residual_kernel<double><<<grid, kRows, smem, s>>>((const double*)X, n, m, k, (const double*)W, (const double*)H, lambda,
                                                           restore, weight, wref, slices, d_partials);

@@ -220,7 +220,7 @@ template <typename T>
 __global__ void __launch_bounds__(256) renormalize_kernel(T* __restrict__ W, T* __restrict__ H, long long n, long long m, int k,
                                                           int normalize) {
     __shared__ double red[8];
-    __shared__ double tot[32];
+    __shared__ double tot[kTiledMaxK];
     const int tid = threadIdx.x, NT = blockDim.x;
     for (int c = 0; c < k; ++c) {
         double s = 0.0;

@@ -53,28 +53,34 @@ __device__ __forceinline__ void tc_stager_role(const TiledPassArgs& a, unsigned 
         offB[q] = 2 * C::B1_BYTES + (col & 7) * 16 + (col >> 3) * C::SBO2 + tb * TC_LBO;
     }
     // ... and of the 16-byte copies of the raw chunk: element offset in V relative to the first step of the unit,
-    // raw index, step within the unit, column in range
+    // raw index, step within the unit, column in range.  K8 > 32: recomputed per copy instead (kept in registers, the tables
+    // of 8 copies spilled to local memory)
     constexpr int NCP = K8 * (TC_TS / 4) / NS;
     static_assert(NCP * NS == K8 * (TC_TS / 4), "copy split");
-    long long cpg[NCP];
-    int cps[NCP], cpt[NCP];
-    bool cpok[NCP];
-#pragma unroll
-    for (int i = 0; i < NCP; ++i) {
+    constexpr bool CPTAB = K8 <= 32;
+    constexpr int NCPT = CPTAB ? NCP : 1;
+    long long cpg[NCPT];
+    int cps[NCPT], cpt[NCPT];
+    bool cpok[NCPT];
+    auto cp_item = [&](int i, long long& g, int& sidx, int& t, bool& ok) {
         const int e = sid + i * NS;
         if (t_major) {
             const int col = e / (TC_TS / 4), t4 = (e % (TC_TS / 4)) * 4;
-            cpg[i] = (long long)t4 + (long long)col * a.sv_a;
-            cps[i] = col * PT + t4;
-            cpt[i] = t4;
-            cpok[i] = col < k;
+            g = (long long)t4 + (long long)col * a.sv_a;
+            sidx = col * PT + t4;
+            t = t4;
+            ok = col < k;
         } else {
             const int tl = e / (K8 / 4), a4 = (e % (K8 / 4)) * 4;
-            cpg[i] = (long long)tl * a.sv_t + a4;
-            cps[i] = tl * PA + a4;
-            cpt[i] = tl;
-            cpok[i] = a4 < k;
+            g = (long long)tl * a.sv_t + a4;
+            sidx = tl * PA + a4;
+            t = tl;
+            ok = a4 < k;
         }
+    };
+    if constexpr (CPTAB) {
+#pragma unroll
+        for (int i = 0; i < NCP; ++i) cp_item(i, cpg[i], cps[i], cpt[i], cpok[i]);
     }
     auto issue_raw = [&](int c, int b, int stage) {
         const float* V = Vg + (long long)s_act[b] * a.v_rstride;
@@ -84,8 +90,16 @@ __device__ __forceinline__ void tc_stager_role(const TiledPassArgs& a, unsigned 
             const float* Vu = V + (long long)t0 * (t_major ? 1 : a.sv_t);
 #pragma unroll
             for (int i = 0; i < NCP; ++i) {
-                const bool live = cpok[i] && (t0 + cpt[i] < t_end);
-                tc::cp_async16_zfill(dst + cps[i], live ? Vu + cpg[i] : V, live ? 16u : 0u);
+                long long g;
+                int sidx, t;
+                bool ok;
+                if constexpr (CPTAB) {
+                    g = cpg[i], sidx = cps[i], t = cpt[i], ok = cpok[i];
+                } else {
+                    cp_item(i, g, sidx, t, ok);
+                }
+                const bool live = ok && (t0 + t < t_end);
+                tc::cp_async16_zfill(dst + sidx, live ? Vu + g : V, live ? 16u : 0u);
             }
         } else {
             for (int e = sid; e < TC_TS * K8; e += NS) {
@@ -186,6 +200,8 @@ __device__ __forceinline__ void tc_stager_role(const TiledPassArgs& a, unsigned 
         if (lane == 0) tc::mbar_arrive(&v_full[vb]);
         if (warp == (first >> 5)) TC_STAMP(2, u, 3);
         if (u + 2 < total) {
+            // two raw buffers (k > 32: shared memory budget): the one refilled below is the one every stager just read
+            if constexpr (C::NRAW < 3) tc::named_bar_sync(1, NS);
             issue_raw(ci, bi, (u + 2) % C::NRAW);
             advance();
         }
