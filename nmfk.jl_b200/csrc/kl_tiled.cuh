@@ -800,6 +800,7 @@ cudaError_t solve_tiled_t(const SolveArgs& a, cudaStream_t s, int64_t* launches)
     int* d_active = nullptr;
     double* fin_tot = nullptr;  // wide finish: the k totals of every restart
     int* fin_flag = nullptr;    //              ... and which restarts tiled_scaleW_kernel has to scale
+    void* vimg = nullptr;       // tcgen05 pass (k <= 16): V operand images, rebuilt before every half-update
     int* h_active = nullptr;  // [0] running restarts, [1] barrier time-out site reported by the tcgen05 kernel
     std::vector<UnitState> hst((size_t)R);
     int it = 0;
@@ -852,6 +853,10 @@ cudaError_t solve_tiled_t(const SolveArgs& a, cudaStream_t s, int64_t* launches)
     NMFK_TRY(scratch_alloc(&d_active, sizeof(int), s));
     NMFK_TRY(scratch_alloc(&fin_tot, (size_t)R * kTiledMaxK * sizeof(double), s));
     NMFK_TRY(scratch_alloc(&fin_flag, (size_t)R * sizeof(int), s));
+    if (use_tc) {
+        const size_t vb = std::max(tc2_image_bytes(k, R, n), tc2_image_bytes(k, R, m));
+        if (vb) NMFK_TRY(scratch_alloc(&vimg, vb, s));
+    }
     h_active = pinned_flags();
     if (h_active == nullptr) NMFK_TRY(cudaErrorMemoryAllocation);
     h_active[0] = h_active[1] = 0;
@@ -867,6 +872,7 @@ cudaError_t solve_tiled_t(const SolveArgs& a, cudaStream_t s, int64_t* launches)
         // restarts of one batch advance in lockstep
         TiledPassArgs ph{}, pw{};
         ph.D = use_td ? a.X : a.Xt;  // the DMMA kernel reads the STEP-contiguous copy, the others the OWN-contiguous one
+        ph.Dstep = a.X;              // ... except the tc2 pass, which reads the step-contiguous one through Dstep
         ph.U = a.H;
         ph.V = a.W;
         ph.den = den;
@@ -890,10 +896,12 @@ cudaError_t solve_tiled_t(const SolveArgs& a, cudaStream_t s, int64_t* launches)
         ph.has_nan = a.has_nan;
         ph.lambda = a.lambda;
         ph.ktmpl = kt;
+        ph.vimg = vimg;
         ph.wait_hint_ns = wait_hint;
         ph.qwait_ns = qwait;
         pw = ph;
         pw.D = use_td ? a.Xt : a.X;
+        pw.Dstep = a.Xt;
         pw.U = a.W;
         pw.V = a.H;
         pw.partial = SW > 1 ? partial : nullptr;
@@ -950,7 +958,7 @@ cudaError_t solve_tiled_t(const SolveArgs& a, cudaStream_t s, int64_t* launches)
                 pt.mark(s, 0);
                 NMFK_TRY((timed_tiled_pass<TX, TC>(ph, red, s, use_tc, h_active + 1, use_td, a.prof)));
                 pt.mark(s, 1);
-                *launches += 2 + (SH > 1 || sharded);
+                *launches += 2 + (SH > 1 || sharded) + (vimg != nullptr);  // + the image producer of the tc2 pass
                 if (d_trace != nullptr) {
                     std::vector<long long> ht(3 * 64 * 8);
                     NMFK_TRY(cudaMemcpyAsync(ht.data(), d_trace, ht.size() * sizeof(long long), cudaMemcpyDeviceToHost, s));
@@ -978,7 +986,7 @@ cudaError_t solve_tiled_t(const SolveArgs& a, cudaStream_t s, int64_t* launches)
                 pt.mark(s, 4);
                 NMFK_TRY((timed_tiled_pass<TX, TC>(pw, nullptr, s, use_tc, h_active + 1, use_td, a.prof)));
                 pt.mark(s, 5);
-                *launches += 2 + (SW > 1);
+                *launches += 2 + (SW > 1) + (vimg != nullptr);
             }
             if (a.has_nan) {
                 dim3 g((n + 127) / 128, R);
@@ -1096,6 +1104,7 @@ done:
     scratch_free(d_active, s);
     scratch_free(fin_tot, s);
     scratch_free(fin_flag, s);
+    scratch_free(vimg, s);
     return err;
 }
 

@@ -28,6 +28,8 @@ struct TiledPassArgs {
     int qwait_ns;          // nanosleep between the quotient warps' polls of p_full (0 = spin)
     long long* trace;   // debug: clock64 stamps of CTA 0 ([role][unit < 64][8]); nullptr in production
     int ktmpl;          // column stride of `partial` (the template K of the combine kernel)
+    const void* Dstep;  // the same data STEP-contiguous: element (o,t) at Dstep[t + o*nred] (tc2 pass: X tiles)
+    void* vimg;         // tc2 pass: scratch for the V operand images, tc2_image_bytes(k, R, nred) bytes
 };
 
 // Float32 half-update on the 5th-generation tensor cores (kl_tiled_tc.cu): tcgen05.mma kind::tf32 with the
@@ -41,6 +43,9 @@ cudaError_t launch_tc_pass(const TiledPassArgs& a, int* d_errflag, cudaStream_t 
 // second generation for k <= 16 (kl_tiled_tc2.cu): U in shared memory, separate P and Q tiles; same grid and arguments
 bool tc2_pass_enabled(int k);
 cudaError_t launch_tc2_pass(const TiledPassArgs& a, int* d_errflag, cudaStream_t s);
+// scratch of the tc2 pass (a.vimg): the V operand images of R restarts over a reduction range of nred steps (0: the pass does
+// not serve k).  A launch first builds the images of its running restarts there, then the pass copies them into shared memory.
+size_t tc2_image_bytes(int k, int R, int nred);
 // one-time host-side set-up (driver entry point of the tensor-map encoder, kernel attributes): called when a context is
 // created so that it never falls inside a timed solve
 void tc2_pass_prepare();

@@ -15,13 +15,19 @@
 //   * TWO threads issue the MMAs (warp 0: MMA#1, warp 1: MMA#2): one thread issuing both spends ~740 clk per unit issuing
 //     (the commit behind the 16 small MMAs of MMA#2 alone costs 75 clk) plus ~450 clk in barrier waits and fences, and was
 //     the critical path of every single-issuer variant;
-//   * X tiles arrive by ONE tensor-map TMA load per chunk (the 64 row-wise bulk copies cost the issuing thread ~2000 clk);
+//   * X tiles arrive by tensor-map TMA loads from the STEP-contiguous copy of the data, two boxes of 128 own indices x 32
+//     steps per chunk, swizzled (SWIZZLE_128B): a quotient thread reads 4 consecutive steps of its own row with one 16-byte
+//     shared load (8 per unit instead of 32 scalar ones), and the 8 threads of a quarter-warp hit 8 different bank groups;
+//   * the V operand images of a unit (hi / lo split, the K-major layouts of MMA#1 and MMA#2, zeros past k and past the last
+//     step) are built once per launch by tc2_images_kernel for every (restart, chunk) and fetched by ONE 1-D bulk copy per
+//     unit; no warp of the pass converts V any more (four stager warps did, and took registers and issue slots from the
+//     quotient warps);
 //   * the numerators of the previous unit are fetched behind the stores of Q and consumed one half-division later.
-// What bounds it now is the quotient stage itself (DESIGN.md 4a): ~5 quotients per clk per SM however it is scheduled.
+// What bounds it now is the quotient stage itself (DESIGN.md 4a).
 //
 // Tensor-memory map (512 columns): P0 | P1 (64 each), Q0 | Q1 (Qhi 64 + Qlo 64 each), two per-unit numerator buffers of 32, U hi of
-// the 4 restarts of the CTA (16 each).  Warps: 0 = MMA#1 issuer, 1 = MMA#2 issuer + TMA producer, 2-5 = V stagers
-// (tc_stage.cuh), 6-21 = two alternating quotient groups.  The objective sums keep using tc_pass_kernel<.., OBJ = true>.
+// the 4 restarts of the CTA (16 each).  Warps: 0 = MMA#1 issuer, 1 = MMA#2 issuer + TMA producer (X tiles and V images),
+// 2-17 = two alternating quotient groups.  The objective sums keep using tc_pass_kernel<.., OBJ = true>.
 #include <algorithm>
 #include <cstdlib>
 #include <mutex>
@@ -41,12 +47,9 @@ struct Tc2Cfg {
     static constexpr int N2 = 16;
     static constexpr int TS = 64;
     static constexpr int NXS = 3;                                     // X tile stages
-    static constexpr int NRAW = 3;                                    // raw V chunk buffers (converting u, u+1 in flight, u+2 issued)
-    static constexpr int NVB = 5;                                     // V image buffers: an image lives from MMA#1(u) to MMA#2(u), ~4 units
-    static constexpr int RPAD = 4;
+    static constexpr int NVB = 6;                                     // V image buffers: an image lives from MMA#1(u) to MMA#2(u), ~4 units
     static constexpr int QW = TS / 4;
-    static constexpr int SW = 4;
-    static constexpr int QW0 = 2 + SW;                                // warps 0, 1: the two MMA issuers
+    static constexpr int QW0 = 2;                                     // warps 0, 1: the two MMA issuers
     static constexpr int THREADS = (QW0 + QW) * 32;
     static constexpr int TCOLS = 512;
     static constexpr int RB = 4;                                      // restarts per CTA (they share the X tiles)
@@ -59,13 +62,10 @@ struct Tc2Cfg {
     static constexpr uint32_t SBO2 = (TS / 4) * 128;
     static constexpr uint32_t B1_BYTES = TS * K8 * 4;
     static constexpr uint32_t B2_BYTES = N2 * TS * 4;
-    static constexpr uint32_t V_BYTES = 2 * B1_BYTES + 2 * B2_BYTES;
-    static constexpr uint32_t X_BYTES = TS * T2_M * 4;
-    static constexpr int RAWP_T = TS + RPAD;
-    static constexpr int RAWP_A = K8 + RPAD;
-    static constexpr uint32_t RAW_BYTES = (K8 * TS + RPAD * (K8 > TS ? K8 : TS)) * 4;
-    static constexpr size_t SMEM =
-        (size_t)NXS * X_BYTES + (size_t)NVB * V_BYTES + (size_t)NRAW * RAW_BYTES + (size_t)RB * U1_BYTES + 32 * 8 + 64;
+    static constexpr uint32_t V_BYTES = 2 * B1_BYTES + 2 * B2_BYTES;  // one unit's images: B1 hi, B1 lo, B2 hi, B2 lo
+    static constexpr uint32_t X_BYTES = TS * T2_M * 4;                // two swizzled boxes of [128 own][32 steps]
+    static constexpr int XBOX = 32;                                   // steps per box: 128 bytes, the swizzle span
+    static constexpr size_t SMEM = (size_t)NXS * X_BYTES + (size_t)NVB * V_BYTES + (size_t)RB * U1_BYTES + 32 * 8 + 64;
     static_assert(SMEM <= 232448, "shared memory budget of one CTA");
 };
 
@@ -80,17 +80,61 @@ __device__ __forceinline__ float rcp_approx(float p) {
     return r;
 }
 
+// V operand images of every running restart r and chunk c of the reduction range (block (c, r)), at
+// vimg + (r * chunks + c) * V_BYTES: B1 = [steps][K8 columns] (MMA#1, K = columns), B2 = [N2 columns][steps] (MMA#2, K = steps),
+// each as hi = the TF32 part and lo = the rest, in the canonical un-swizzled K-major layout.  Item it = 16 bytes = 4 values at
+// byte it * 16 of its image (8 rows x 16 bytes per core matrix, core matrices along K first), so a warp writes 512 contiguous bytes.
+template <int K8>
+__global__ void __launch_bounds__(256) tc2_images_kernel(const TiledPassArgs a, int chunks) {
+    using C = Tc2Cfg<K8>;
+    const int c = blockIdx.x, r = blockIdx.y;
+    if (a.st[r].stop != 0) return;  // frozen: the pass does not read it
+    const float* V = static_cast<const float*>(a.V) + (long long)r * a.v_rstride;
+    float4* img = reinterpret_cast<float4*>(static_cast<unsigned char*>(a.vimg) + ((size_t)r * chunks + c) * C::V_BYTES);
+    const int t0 = c * C::TS;
+    auto val = [&](int t, int col) {
+        return (t0 + t < a.nred && col < a.k) ? V[(long long)(t0 + t) * a.sv_t + (long long)col * a.sv_a] : 0.f;
+    };
+    constexpr int NAB = K8 / 4, NTB = C::TS / 4;
+    constexpr int NA = C::TS * NAB, NB = C::N2 * NTB;
+    for (int it = threadIdx.x; it < NA + NB; it += blockDim.x) {
+        float v[4];
+        int hi, lo;
+        if (it < NA) {  // B1: row = step t, 4 columns 4 ab ..
+            const int t = (it & 7) + 8 * (it / (8 * NAB)), ab = (it >> 3) % NAB;
+#pragma unroll
+            for (int j = 0; j < 4; ++j) v[j] = val(t, ab * 4 + j);
+            hi = it;
+            lo = it + C::B1_BYTES / 16;
+        } else {  // B2: row = column, 4 steps 4 tb ..
+            const int ib = it - NA;
+            const int col = (ib & 7) + 8 * (ib / (8 * NTB)), tb = (ib >> 3) % NTB;
+#pragma unroll
+            for (int i = 0; i < 4; ++i) v[i] = val(tb * 4 + i, col);
+            hi = 2 * C::B1_BYTES / 16 + ib;
+            lo = hi + C::B2_BYTES / 16;
+        }
+        float h[4], l[4];
+#pragma unroll
+        for (int j = 0; j < 4; ++j) {
+            h[j] = __uint_as_float(__float_as_uint(v[j]) & 0xffffe000u);
+            l[j] = v[j] - h[j];
+        }
+        img[hi] = make_float4(h[0], h[1], h[2], h[3]);
+        img[lo] = make_float4(l[0], l[1], l[2], l[3]);
+    }
+}
+
 template <int K8>
 __global__ void __launch_bounds__((Tc2Cfg<K8>::THREADS), 1) tc2_pass_kernel(const TiledPassArgs a, const __grid_constant__ CUtensorMap mX,
                                                                             int* errflag) {
     using C = Tc2Cfg<K8>;
-    constexpr int NXS = C::NXS, NVB = C::NVB, TS = C::TS, QWARPS = C::QW, SWARPS = C::SW, QW0 = C::QW0, THREADS = C::THREADS;
+    constexpr int NXS = C::NXS, NVB = C::NVB, TS = C::TS, QWARPS = C::QW, QW0 = C::QW0;
     constexpr int RB = C::RB, N2 = C::N2;
     extern __shared__ __align__(1024) unsigned char smem[];
-    float* Xs = reinterpret_cast<float*>(smem);                                   // [NXS][TS][M]
+    float* Xs = reinterpret_cast<float*>(smem);                                   // [NXS][2][M][XBOX] (swizzled)
     unsigned char* Vs = smem + (size_t)NXS * C::X_BYTES;                           // [NVB][V_BYTES]
-    float* Raw = reinterpret_cast<float*>(Vs + (size_t)NVB * C::V_BYTES);          // [NRAW][RAW_BYTES]
-    unsigned char* Us = reinterpret_cast<unsigned char*>(Raw) + (size_t)C::NRAW * C::RAW_BYTES;  // [RB] U lo images
+    unsigned char* Us = Vs + (size_t)NVB * C::V_BYTES;                             // [RB] U lo images
     uint64_t* bars = reinterpret_cast<uint64_t*>(Us + (size_t)RB * C::U1_BYTES);
     uint64_t* x_full = bars;             // [NXS]
     uint64_t* x_empty = x_full + NXS;    // [NXS]
@@ -104,7 +148,6 @@ __global__ void __launch_bounds__((Tc2Cfg<K8>::THREADS), 1) tc2_pass_kernel(cons
     int* s_act = reinterpret_cast<int*>(tmem_slot + 1);
 
     const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
-    const uint32_t hint = (uint32_t)a.wait_hint_ns;
     long long* const trc = (a.trace != nullptr && blockIdx.x == 0) ? a.trace : nullptr;
     const int ngroups = (a.R + RB - 1) / RB;
     const int g = blockIdx.x % ngroups;
@@ -113,7 +156,7 @@ __global__ void __launch_bounds__((Tc2Cfg<K8>::THREADS), 1) tc2_pass_kernel(cons
     const int slice = rest / a.nblocks;
     const int o0 = ob * T2_M;
     const int k = a.k;
-    const int chunks_all = (a.nred + TS - 1) / TS;
+    const int chunks_all = (a.nred + TS - 1) / TS;  // chunks of the whole reduction range (the image scratch is indexed by them)
     const int t_begin = (int)(((long long)chunks_all * slice) / a.S) * TS;
     const int t_end = min(a.nred, (int)(((long long)chunks_all * (slice + 1)) / a.S) * TS);
     const int nchunks = (t_end - t_begin + TS - 1) / TS;
@@ -141,7 +184,7 @@ __global__ void __launch_bounds__((Tc2Cfg<K8>::THREADS), 1) tc2_pass_kernel(cons
             tc::mbar_init(&x_empty[i], QWARPS);
         }
         for (int i = 0; i < NVB; ++i) {
-            tc::mbar_init(&v_full[i], SWARPS);
+            tc::mbar_init(&v_full[i], 1);
             tc::mbar_init(&v_empty[i], 1);
         }
         for (int i = 0; i < 2; ++i) {
@@ -152,7 +195,6 @@ __global__ void __launch_bounds__((Tc2Cfg<K8>::THREADS), 1) tc2_pass_kernel(cons
         }
         tc::mbar_fence_init();
     }
-    for (uint32_t e = tid; e < NVB * C::V_BYTES / 16; e += THREADS) reinterpret_cast<uint4*>(Vs)[e] = make_uint4(0, 0, 0, 0);
     if (tid == 0) tma_prefetch_map(&mX);
 
     float* Ug = static_cast<float*>(a.U);
@@ -233,8 +275,10 @@ __global__ void __launch_bounds__((Tc2Cfg<K8>::THREADS), 1) tc2_pass_kernel(cons
         }
         __syncwarp();
     } else if (warp == 1) {
-        // ===== MMA#2 issuer + TMA producer: ACC(u) = Q(u) V once Q(u) is stored; one tensor-map TMA load per X tile (box = 128
-        // own indices x 64 steps, zero fill past the edges of X) - chunk c+NXS as soon as both groups are through chunk c =====
+        // ===== MMA#2 issuer + TMA producer: ACC(u) = Q(u) V once Q(u) is stored; two tensor-map TMA loads per X tile (boxes of
+        // 32 steps x 128 own indices, zero fill past the edges of X) - chunk c+NXS as soon as both groups are through chunk c;
+        // one bulk copy per unit of its V images into the ring - unit w as soon as MMA#2 of unit w-NVB is done with the
+        // buffer: unit u+NVB-2 for certain before waiting for Q(u), unit u+NVB-1 if MMA#2(u-1) is already through =====
         constexpr uint32_t idA1 = tc::idesc_tf32(T2_M, C::ACOLS, 0);
         constexpr uint32_t idA2 = tc::idesc_tf32(T2_M, N2, 0);
         const uint64_t d2 = tc::smem_desc(tc::smem_u32(Vs) + 2 * C::B1_BYTES, TC_LBO, C::SBO2);
@@ -243,15 +287,33 @@ __global__ void __launch_bounds__((Tc2Cfg<K8>::THREADS), 1) tc2_pass_kernel(cons
             const int s = c % NXS;
             if (tc::elect_one()) {
                 tc::mbar_arrive_expect_tx(&x_full[s], C::X_BYTES);
-                tma_load_2d(Xs + (size_t)s * TS * T2_M, &mX, o0, t_begin + c * TS, &x_full[s]);
+                tma_load_2d(Xs + (size_t)s * TS * T2_M, &mX, t_begin + c * TS, o0, &x_full[s]);
+                tma_load_2d(Xs + (size_t)s * TS * T2_M + C::XBOX * T2_M, &mX, t_begin + c * TS + C::XBOX, o0, &x_full[s]);
             }
             __syncwarp();
         };
         for (int c = 0; c < NXS && c < nchunks; ++c) load_x(c);
+        const unsigned char* vimg = static_cast<const unsigned char*>(a.vimg) + (size_t)(t_begin / TS) * C::V_BYTES;
+        auto load_v = [&](int w) {
+            const int vb = w % NVB, c = w / nact;
+            if (tc::elect_one()) {
+                tc::mbar_arrive_expect_tx(&v_full[vb], C::V_BYTES);
+                tc::bulk_g2s(Vs + (size_t)vb * C::V_BYTES, vimg + ((size_t)s_act[w - c * nact] * chunks_all + c) * C::V_BYTES, C::V_BYTES,
+                             &v_full[vb]);
+            }
+            __syncwarp();
+        };
+        auto v_released = [&](int w) { return &v_empty[w % NVB]; };  // ... by MMA#2 of unit w - NVB: phase (w / NVB - 1) & 1
+        int vnext = 0;                                                // next unit whose images are to be fetched
+        for (; vnext < NVB && vnext < total; ++vnext) load_v(vnext);
         int cdone = 0, ub = 0;  // chunks whose last MMA#2 has been issued; u % nact
         int xwait = -1;         // chunk whose stage the next X load waits for (-1: none pending)
         for (int u = 0; u < total; ++u) {
             const int vb = u % NVB;
+            for (; vnext < total && vnext <= u + NVB - 2; ++vnext) {
+                tc::mbar_wait_h(0u, v_released(vnext), (uint32_t)((vnext / NVB - 1) & 1), errflag, 22);
+                load_v(vnext);
+            }
             TC_STAMP(1, u, 0);
             tc::mbar_wait_h(0u, &q_full[u & 1], (uint32_t)((u >> 1) & 1), errflag, 21);
             tc::tc_fence_after_sync();
@@ -269,6 +331,10 @@ __global__ void __launch_bounds__((Tc2Cfg<K8>::THREADS), 1) tc2_pass_kernel(cons
             }
             __syncwarp();
             TC_STAMP(1, u, 2);
+            if (vnext < total && vnext == u + NVB - 1 && tc::mbar_test(v_released(vnext), (uint32_t)((vnext / NVB - 1) & 1))) {
+                load_v(vnext);
+                ++vnext;
+            }
             if (xwait >= 0 && tc::mbar_test(&x_empty[xwait % NXS], (uint32_t)((xwait / NXS) & 1))) {
                 load_x(xwait + NXS);
                 xwait = -1;
@@ -285,8 +351,6 @@ __global__ void __launch_bounds__((Tc2Cfg<K8>::THREADS), 1) tc2_pass_kernel(cons
             }
         }
         __syncwarp();
-    } else if (warp < QW0) {
-        tc_stager_role<C, K8, false>(a, Vs, Raw, v_full, v_empty, s_act, nact, total, t_begin, t_end, 64, hint, errflag, trc);
     } else {
         // ===== quotient warps: two GROUPS of 8 warps (4 lane quarters x 2 column halves of 32) alternate units =====
         const int lq = warp & 3, cs = (warp - QW0) >> 2;
@@ -317,12 +381,16 @@ __global__ void __launch_bounds__((Tc2Cfg<K8>::THREADS), 1) tc2_pass_kernel(cons
         };
         const uint32_t pcol = lane_base + C::PBASE + (uint32_t)grp * TS + jh;
         const uint32_t qcol = lane_base + C::QBASE + (uint32_t)grp * 2 * TS + jh;
+        // X row of this thread in each stage: box hh (steps jh .. jh+31), 128 bytes at o_loc; 16-byte piece i of the row (steps
+        // jh+4i .. jh+4i+3) sits at piece i ^ (address bits 7-9), the SWIZZLE_128B pattern of the TMA load
+        const uint32_t xrow = (uint32_t)(hh * C::XBOX * T2_M + o_loc * C::XBOX) * 4;
+        const uint32_t xsw = ((tc::smem_u32(Xs) + xrow) >> 7) & 7;
         int prev_slot = -1;
         for (int c = 0; c < nchunks; ++c) {
             const int s = c % NXS;
             const int cnt = min(TS, t_end - (t_begin + c * TS));
             tc::mbar_wait_h(0u, &x_full[s], (uint32_t)((c / NXS) & 1), errflag, 40);
-            const float* xs = Xs + (size_t)s * TS * T2_M + (size_t)jh * T2_M + o_loc;
+            const unsigned char* xs = reinterpret_cast<const unsigned char*>(Xs + (size_t)s * TS * T2_M) + xrow;
             for (int b = grp; b < nact; b += 2) {
                 const int u = c * nact + b;  // u % 2 == grp (nact is even)
                 if (warp == QW0) TC_STAMP(0, u, 0);
@@ -341,7 +409,12 @@ __global__ void __launch_bounds__((Tc2Cfg<K8>::THREADS), 1) tc2_pass_kernel(cons
                     }
                     if (half == 0 && warp == QW0) TC_STAMP(0, u, 2);
                     uint32_t lo[16];
-                    const float* xh = xs + half * 16 * T2_M;
+                    float xv[16];
+#pragma unroll
+                    for (int i = 0; i < 4; ++i) {
+                        const float4 x4 = *reinterpret_cast<const float4*>(xs + (((uint32_t)(half * 4 + i) ^ xsw) << 4));
+                        xv[4 * i] = x4.x, xv[4 * i + 1] = x4.y, xv[4 * i + 2] = x4.z, xv[4 * i + 3] = x4.w;
+                    }
                     if (cnt == TS) {
 #pragma unroll
                         for (int j = 0; j < 16; j += 2) {
@@ -350,7 +423,7 @@ __global__ void __launch_bounds__((Tc2Cfg<K8>::THREADS), 1) tc2_pass_kernel(cons
                             // stage - and p0 p1 underflows for the tiny products of all-zero rows.)
                             const int jj = j;
                             const float r0 = rcp_approx(__uint_as_float(p[jj])), r1 = rcp_approx(__uint_as_float(p[jj + 1]));
-                            const unsigned long long x2 = pack2f(xh[j * T2_M], xh[(j + 1) * T2_M]), r2 = pack2f(r0, r1);
+                            const unsigned long long x2 = pack2f(xv[j], xv[j + 1]), r2 = pack2f(r0, r1);
                             unsigned long long q2, l2;
                             asm("mul.rn.f32x2 %0, %1, %2;" : "=l"(q2) : "l"(x2), "l"(r2));
                             const unsigned long long h2 = q2 & 0xffffe000ffffe000ull;
@@ -364,7 +437,7 @@ __global__ void __launch_bounds__((Tc2Cfg<K8>::THREADS), 1) tc2_pass_kernel(cons
 #pragma unroll
                         for (int j = 0; j < 16; ++j) {
                             const int jj = j;
-                            float q = xh[j * T2_M] * rcp_approx(__uint_as_float(p[jj]));
+                            float q = xv[j] * rcp_approx(__uint_as_float(p[jj]));
                             q = (jh + half * 16 + jj < cnt) ? q : 0.f;
                             const uint32_t h = __float_as_uint(q) & 0xffffe000u;
                             lo[j] = __float_as_uint(q - __uint_as_float(h));
@@ -454,11 +527,12 @@ cudaError_t launch2(const TiledPassArgs& a, int* d_errflag, cudaStream_t s) {
     using C = Tc2Cfg<K8>;
     const int ngroups = (a.R + C::RB - 1) / C::RB;
     const long long grid = (long long)a.S * a.nblocks * ngroups;
-    if (grid > 2147483647ll) return cudaErrorInvalidValue;
+    const int chunks = (a.nred + C::TS - 1) / C::TS;
+    if (grid > 2147483647ll || a.vimg == nullptr || a.R > 65535) return cudaErrorInvalidValue;
     cudaError_t e = cudaFuncSetAttribute(tc2_pass_kernel<K8>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)C::SMEM);
     if (e != cudaSuccess) return e;
-    // D: element (own o, step t) at D[o + t * nown].  The map is a pure function of (D, nown, nred): the two maps of a solve
-    // (X and its transpose) are encoded once and reused by every launch.
+    // Dstep: element (own o, step t) at Dstep[t + o * nred].  The map is a pure function of (Dstep, nown, nred): the two maps of
+    // a solve (X and its transpose) are encoded once and reused by every launch.
     struct Cached {
         const void* base;
         int nown, nred;
@@ -472,19 +546,22 @@ cudaError_t launch2(const TiledPassArgs& a, int* d_errflag, cudaStream_t s) {
         std::lock_guard<std::mutex> lock(mu);
         int hit = -1;
         for (int i = 0; i < 4; ++i)
-            if (cache[i].base == a.D && cache[i].nown == a.nown && cache[i].nred == a.nred) hit = i;
+            if (cache[i].base == a.Dstep && cache[i].nown == a.nown && cache[i].nred == a.nred) hit = i;
         if (hit < 0) {
             hit = next;
             next = (next + 1) % 4;
             cache[hit].base = nullptr;
-            if (!tma_make_map_f32(&cache[hit].map, a.D, a.nown, a.nred, a.nown, T2_M, C::TS, CU_TENSOR_MAP_SWIZZLE_NONE))
+            if (!tma_make_map_f32(&cache[hit].map, a.Dstep, a.nred, a.nown, a.nred, C::XBOX, T2_M, CU_TENSOR_MAP_SWIZZLE_128B))
                 return cudaErrorNotSupported;
-            cache[hit].base = a.D;
+            cache[hit].base = a.Dstep;
             cache[hit].nown = a.nown;
             cache[hit].nred = a.nred;
         }
         mX = cache[hit].map;
     }
+    tc2_images_kernel<K8><<<dim3((unsigned)chunks, (unsigned)a.R), 256, 0, s>>>(a, chunks);
+    e = cudaGetLastError();
+    if (e != cudaSuccess) return e;
     tc2_pass_kernel<K8><<<(unsigned)grid, C::THREADS, C::SMEM, s>>>(a, mX, d_errflag);
     return cudaGetLastError();
 }
@@ -500,6 +577,12 @@ bool tc2_pass_enabled(int k) {
     return gen >= 2 && k <= 16 && tma_encode_fn() != nullptr;
 }
 
+size_t tc2_image_bytes(int k, int R, int nred) {
+    const size_t per = k <= 8 ? Tc2Cfg<8>::V_BYTES : Tc2Cfg<16>::V_BYTES;
+    constexpr int TS = Tc2Cfg<16>::TS;
+    return tc2_pass_enabled(k) ? (size_t)R * (size_t)((nred + TS - 1) / TS) * per : 0;
+}
+
 void tc2_pass_prepare() {
     static bool done = false;
     if (done) return;
@@ -507,7 +590,7 @@ void tc2_pass_prepare() {
     CUtensorMap m;  // a first (dummy) encode and the function look-ups: the driver does lazy work on both
     float* dummy = nullptr;
     if (cudaMalloc(&dummy, 1 << 20) == cudaSuccess) {
-        (void)tma_make_map_f32(&m, dummy, 512, 512, 512, T2_M, 64, CU_TENSOR_MAP_SWIZZLE_NONE);
+        (void)tma_make_map_f32(&m, dummy, 512, 512, 512, 32, T2_M, CU_TENSOR_MAP_SWIZZLE_128B);
         cudaFree(dummy);
     }
     cudaFuncAttributes fa;

@@ -1,4 +1,4 @@
-// V stager role of the tcgen05 tiled passes (kl_tiled_tc.cu, kl_tiled_tc2.cu): 128 threads cp.async the raw chunk of the
+// V stager role of the first-generation tcgen05 tiled pass (kl_tiled_tc.cu): 128 threads cp.async the raw chunk of the
 // broadcast factor two units ahead (16 bytes at a time along whichever index is contiguous in global memory), then split it
 // hi / lo (TF32 + rest) into the two canonical un-swizzled K-major images that MMA#1 (rows = steps, K = columns) and MMA#2
 // (rows = columns, K = steps) read.  Work item = half a 4 x 4 block.
