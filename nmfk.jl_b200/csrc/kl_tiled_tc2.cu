@@ -15,6 +15,9 @@
 //   * TWO threads issue the MMAs (warp 0: MMA#1, warp 1: MMA#2): one thread issuing both spends ~740 clk per unit issuing
 //     (the commit behind the 16 small MMAs of MMA#2 alone costs 75 clk) plus ~450 clk in barrier waits and fences, and was
 //     the critical path of every single-issuer variant;
+//   * a THIRD thread (warp 18) does all the loading, so the MMA#2 thread only waits for Q: with the X and V loads and
+//     their barrier waits on it as well, it reached each unit ~1300 clk after Q was stored, and the quotient groups waited
+//     for its a_full (profiles/r05_tc2_trace_c3_main.txt);
 //   * X tiles arrive by tensor-map TMA loads from the STEP-contiguous copy of the data, two boxes of 128 own indices x 32
 //     steps per chunk, swizzled (SWIZZLE_128B): a quotient thread reads 4 consecutive steps of its own row with one 16-byte
 //     shared load (8 per unit instead of 32 scalar ones), and the 8 threads of a quarter-warp hit 8 different bank groups;
@@ -26,8 +29,9 @@
 // What bounds it now is the quotient stage itself (DESIGN.md 4a).
 //
 // Tensor-memory map (512 columns): P0 | P1 (64 each), Q0 | Q1 (Qhi 64 + Qlo 64 each), two per-unit numerator buffers of 32, U hi of
-// the 4 restarts of the CTA (16 each).  Warps: 0 = MMA#1 issuer, 1 = MMA#2 issuer + TMA producer (X tiles and V images),
-// 2-17 = two alternating quotient groups.  The objective sums keep using tc_pass_kernel<.., OBJ = true>.
+// the 4 restarts of the CTA (16 each).  Warps: 0 = MMA#1 issuer, 1 = MMA#2 issuer, 2-17 = two alternating quotient groups,
+// 18 = load warp (X tiles and V images; last, because a warp reaches only the tensor-memory lanes of its warp % 4 quarter and
+// this one touches none).  The objective sums keep using tc_pass_kernel<.., OBJ = true>.
 #include <algorithm>
 #include <cstdlib>
 #include <mutex>
@@ -50,7 +54,8 @@ struct Tc2Cfg {
     static constexpr int NVB = 6;                                     // V image buffers: an image lives from MMA#1(u) to MMA#2(u), ~4 units
     static constexpr int QW = TS / 4;
     static constexpr int QW0 = 2;                                     // warps 0, 1: the two MMA issuers
-    static constexpr int THREADS = (QW0 + QW) * 32;
+    static constexpr int LW = QW0 + QW;                               // the load warp, after the quotient warps
+    static constexpr int THREADS = (LW + 1) * 32;
     static constexpr int TCOLS = 512;
     static constexpr int RB = 4;                                      // restarts per CTA (they share the X tiles)
     static constexpr int ACOLS = 2 * N2;                              // Qhi * [Vhi ; Vlo] stacked along N
@@ -208,7 +213,7 @@ __global__ void __launch_bounds__((Tc2Cfg<K8>::THREADS), 1) tc2_pass_kernel(cons
     // own factor rows, split hi / lo: hi -> tensor memory, lo -> the canonical K-major image in shared memory (the A operands
     // of MMA#1); quotient warp column group cs loads restart slot cs.  Own indices past the edge get U = 1 (finite P; their X
     // is 0 and their rows are never stored).
-    if (warp >= QW0) {
+    if (warp >= QW0 && warp < C::LW) {
         const int lq = warp & 3, cs = (warp - QW0) >> 2;
         const int ol = lq * 32 + lane;
         const int o = o0 + ol;
@@ -275,51 +280,21 @@ __global__ void __launch_bounds__((Tc2Cfg<K8>::THREADS), 1) tc2_pass_kernel(cons
         }
         __syncwarp();
     } else if (warp == 1) {
-        // ===== MMA#2 issuer + TMA producer: ACC(u) = Q(u) V once Q(u) is stored; two tensor-map TMA loads per X tile (boxes of
-        // 32 steps x 128 own indices, zero fill past the edges of X) - chunk c+NXS as soon as both groups are through chunk c;
-        // one bulk copy per unit of its V images into the ring - unit w as soon as MMA#2 of unit w-NVB is done with the
-        // buffer: unit u+NVB-2 for certain before waiting for Q(u), unit u+NVB-1 if MMA#2(u-1) is already through =====
+        // ===== MMA#2 issuer: ACC(u) = Q(u) V as soon as Q(u) is stored.  Nothing else: every clk this thread spends elsewhere
+        // delays a_full(u), and with it the quotient group's first store of Q(u+2) =====
         constexpr uint32_t idA1 = tc::idesc_tf32(T2_M, C::ACOLS, 0);
         constexpr uint32_t idA2 = tc::idesc_tf32(T2_M, N2, 0);
         const uint64_t d2 = tc::smem_desc(tc::smem_u32(Vs) + 2 * C::B1_BYTES, TC_LBO, C::SBO2);
         constexpr uint64_t KSTEP = (2 * TC_LBO) >> 4;
-        auto load_x = [&](int c) {
-            const int s = c % NXS;
-            if (tc::elect_one()) {
-                tc::mbar_arrive_expect_tx(&x_full[s], C::X_BYTES);
-                tma_load_2d(Xs + (size_t)s * TS * T2_M, &mX, t_begin + c * TS, o0, &x_full[s]);
-                tma_load_2d(Xs + (size_t)s * TS * T2_M + C::XBOX * T2_M, &mX, t_begin + c * TS + C::XBOX, o0, &x_full[s]);
-            }
-            __syncwarp();
-        };
-        for (int c = 0; c < NXS && c < nchunks; ++c) load_x(c);
-        const unsigned char* vimg = static_cast<const unsigned char*>(a.vimg) + (size_t)(t_begin / TS) * C::V_BYTES;
-        auto load_v = [&](int w) {
-            const int vb = w % NVB, c = w / nact;
-            if (tc::elect_one()) {
-                tc::mbar_arrive_expect_tx(&v_full[vb], C::V_BYTES);
-                tc::bulk_g2s(Vs + (size_t)vb * C::V_BYTES, vimg + ((size_t)s_act[w - c * nact] * chunks_all + c) * C::V_BYTES, C::V_BYTES,
-                             &v_full[vb]);
-            }
-            __syncwarp();
-        };
-        auto v_released = [&](int w) { return &v_empty[w % NVB]; };  // ... by MMA#2 of unit w - NVB: phase (w / NVB - 1) & 1
-        int vnext = 0;                                                // next unit whose images are to be fetched
-        for (; vnext < NVB && vnext < total; ++vnext) load_v(vnext);
-        int cdone = 0, ub = 0;  // chunks whose last MMA#2 has been issued; u % nact
-        int xwait = -1;         // chunk whose stage the next X load waits for (-1: none pending)
+        int vb = 0;  // u % NVB
         for (int u = 0; u < total; ++u) {
-            const int vb = u % NVB;
-            for (; vnext < total && vnext <= u + NVB - 2; ++vnext) {
-                tc::mbar_wait_h(0u, v_released(vnext), (uint32_t)((vnext / NVB - 1) & 1), errflag, 22);
-                load_v(vnext);
-            }
+            const uint32_t h = (uint32_t)(u & 1);
             TC_STAMP(1, u, 0);
-            tc::mbar_wait_h(0u, &q_full[u & 1], (uint32_t)((u >> 1) & 1), errflag, 21);
+            tc::mbar_wait_h(0u, &q_full[h], (uint32_t)((u >> 1) & 1), errflag, 21);
             tc::tc_fence_after_sync();
             TC_STAMP(1, u, 1);
-            const uint32_t d = tbase + C::ABASE + (uint32_t)(u & 1) * C::ACOLS;
-            const uint32_t qh = tbase + C::QBASE + (uint32_t)(u & 1) * 2 * TS, ql = qh + TS;
+            const uint32_t d = tbase + C::ABASE + h * C::ACOLS;
+            const uint32_t qh = tbase + C::QBASE + h * 2 * TS, ql = qh + TS;
             const uint64_t bh = d2 + (uint64_t)((vb * C::V_BYTES) >> 4);
             if (tc::elect_one()) {
 #pragma unroll
@@ -327,27 +302,68 @@ __global__ void __launch_bounds__((Tc2Cfg<K8>::THREADS), 1) tc2_pass_kernel(cons
 #pragma unroll
                 for (int ks = 0; ks < TS / 8; ++ks) tc::mma_tf32_ts(d, ql + ks * 8, bh + ks * KSTEP, idA2, 1);
                 tc::mma_commit(&v_empty[vb]);
-                tc::mma_commit(&a_full[u & 1]);
+                tc::mma_commit(&a_full[h]);
             }
             __syncwarp();
             TC_STAMP(1, u, 2);
-            if (vnext < total && vnext == u + NVB - 1 && tc::mbar_test(v_released(vnext), (uint32_t)((vnext / NVB - 1) & 1))) {
-                load_v(vnext);
-                ++vnext;
+            vb = vb + 1 == NVB ? 0 : vb + 1;
+        }
+        __syncwarp();
+    } else if (warp == C::LW) {
+        // ===== load warp, in unit order: before the first unit of chunk c its X tile (two tensor-map TMA loads, boxes of 32
+        // steps x 128 own indices, zero fill past the edges of X) once both groups are through chunk c-NXS, the previous user
+        // of the stage; then the V images of each unit w (one bulk copy into the ring) once MMA#2(w-NVB) is done with the
+        // buffer.
+        // Deadlock-freedom: every role handles its units in increasing order, and every wait is for a stage of an earlier
+        // unit or of an earlier step of the same unit, so the lowest unfinished unit can always progress.  The waits:
+        //   load warp  V(w): v_empty = MMA#2(w-NVB) done.  X(c): x_empty = both groups through the units of chunk c-NXS, all
+        //              below c*nact, the unit it loads next (X(c) goes out before V(c*nact), so a group never waits for an X
+        //              tile behind a V wait of a later unit);
+        //   MMA#1(u)   p_empty = the group has P(u-2) in registers; v_full = V(u) loaded;
+        //   MMA#2(u)   q_full = Q(u) stored;
+        //   group, u   x_full of its chunk, p_full = MMA#1(u) done, a_full = MMA#2(u-2) done.
+        // The edge cases keep this order:
+        //   * nact = 2 with the shadow unit: nact counts it, so all roles see the same total = nchunks * nact units and the same
+        //     chunk boundaries; the shadow unit loads the images of slot 0 again, and its numerators are never stored;
+        //   * nchunks < NXS: only nchunks tiles are loaded and no x_empty is waited for; the arrivals on them are never awaited;
+        //   * slices (S > 1): every role counts its chunks from the same [t_begin, t_end), the images from chunk t_begin / TS;
+        //   * restarts frozen by stop are left out of s_act before any role starts, and a CTA with none running returns before
+        //     the barriers are initialised. =====
+        auto load_x = [&](int c, int s) {
+            if (tc::elect_one()) {
+                tc::mbar_arrive_expect_tx(&x_full[s], C::X_BYTES);
+                tma_load_2d(Xs + (size_t)s * TS * T2_M, &mX, t_begin + c * TS, o0, &x_full[s]);
+                tma_load_2d(Xs + (size_t)s * TS * T2_M + C::XBOX * T2_M, &mX, t_begin + c * TS + C::XBOX, o0, &x_full[s]);
             }
-            if (xwait >= 0 && tc::mbar_test(&x_empty[xwait % NXS], (uint32_t)((xwait / NXS) & 1))) {
-                load_x(xwait + NXS);
-                xwait = -1;
+            __syncwarp();
+        };
+        for (int c = 0; c < NXS && c < nchunks; ++c) load_x(c, c);
+        const unsigned char* vimg = static_cast<const unsigned char*>(a.vimg) + (size_t)(t_begin / TS) * C::V_BYTES;
+        int c = 0, b = 0, s = 0;  // chunk of unit w, w % nact, c % NXS
+        int vb = 0, vround = 0;   // w % NVB, w / NVB
+        for (int w = 0; w < total; ++w) {
+            if (b == 0 && c >= NXS) {
+                TC_STAMP(2, w, 4);
+                tc::mbar_wait_h(0u, &x_empty[s], (uint32_t)((c / NXS - 1) & 1), errflag, 10);
+                TC_STAMP(2, w, 5);
+                load_x(c, s);
+                TC_STAMP(2, w, 6);
             }
-            ub = ub + 1 == nact ? 0 : ub + 1;
-            if (ub == 0) {  // unit u was the last one of chunk cdone: both groups are through its X tile (or about to be)
-                if (xwait >= 0) {
-                    tc::mbar_wait_h(0u, &x_empty[xwait % NXS], (uint32_t)((xwait / NXS) & 1), errflag, 10);
-                    load_x(xwait + NXS);
-                    xwait = -1;
-                }
-                if (cdone + NXS < nchunks) xwait = cdone;
-                ++cdone;
+            TC_STAMP(2, w, 0);
+            if (vround > 0) tc::mbar_wait_h(0u, &v_empty[vb], (uint32_t)((vround - 1) & 1), errflag, 22);
+            TC_STAMP(2, w, 1);
+            if (tc::elect_one()) {
+                tc::mbar_arrive_expect_tx(&v_full[vb], C::V_BYTES);
+                tc::bulk_g2s(Vs + (size_t)vb * C::V_BYTES, vimg + ((size_t)s_act[b] * chunks_all + c) * C::V_BYTES, C::V_BYTES,
+                             &v_full[vb]);
+            }
+            __syncwarp();
+            TC_STAMP(2, w, 2);
+            if (++vb == NVB) vb = 0, ++vround;
+            if (++b == nact) {
+                b = 0;
+                ++c;
+                s = s + 1 == NXS ? 0 : s + 1;
             }
         }
         __syncwarp();
