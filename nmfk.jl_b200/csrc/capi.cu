@@ -737,6 +737,7 @@ static void fill_args(const nmfk_batch* b, const nmfk_params* p, SolveArgs& a) {
     a.tiled_tc = p->engine != NMFK_ENGINE_TILED_SCALAR;
     a.shard = c->sharded ? &c->shard : nullptr;
     a.prof = c->prof.enabled ? const_cast<PassProfile*>(&c->prof) : nullptr;
+    a.timeout = nullptr;
 }
 
 // tiled engine (kl_tiled.cu): host-driven, for factors that do not fit in shared memory
@@ -744,6 +745,17 @@ namespace nmfk {
 cudaError_t solve_tiled(const SolveArgs& a, int dtype, cudaStream_t s, int64_t* launches);
 bool tiled_supported(int k);
 }  // namespace nmfk
+
+// a solver's return value; a barrier time-out it reported becomes an error naming the kernel and the site, like nmfk_gemm_nt's
+// (status: the CUDA error of the trap that ends the time-out when the solver met it, NMFK_E_INVALID otherwise)
+static int32_t solve_status(nmfk_ctx* c, const char* solver, cudaError_t e, const KernelTimeout& to) {
+    if (to.kernel != nullptr)
+        return fail(c, e == cudaErrorLaunchTimeout ? NMFK_E_INVALID : (int32_t)e,
+                    std::string(solver) + ": barrier time-out inside " + to.kernel + " (" + to.where + ", site " + std::to_string(to.site) +
+                        "): " + cudaGetErrorString(e));
+    CU(c, e);
+    return NMFK_OK;
+}
 
 // Epilogue of NMFmultiplicative with a normalizevector (NMFkMultiplicative.jl:119-125) followed by the objective / normalisation
 // of execute_singlerun_compute (NMFkExecute.jl:791-804), for the restarts an engine has just finished (done == 1) on the
@@ -800,7 +812,10 @@ static int32_t solve_fro_batches(nmfk_ctx* c, nmfk_batch* const* batches, int32_
         if (batches[i]->k > 32) return fail(c, NMFK_E_UNSUPPORTED, "variant FRO: k > 32 is not supported");
         SolveArgs a;
         fill_args(batches[i], p, a);
-        CU(c, solve_fro(a, c->dtype, c->Xlo, c->Xtlo, c->stream, &c->launches));
+        KernelTimeout to;
+        a.timeout = &to;
+        const int32_t rc = solve_status(c, "variant FRO", solve_fro(a, c->dtype, c->Xlo, c->Xtlo, c->stream, &c->launches), to);
+        if (rc) return rc;
     }
     CU(c, cudaEventRecord(c->ev1, c->stream));
     CU(c, cudaEventSynchronize(c->ev1));
@@ -916,7 +931,12 @@ int32_t nmfk_solve(nmfk_ctx* c, nmfk_batch* const* batches, int32_t nb, const nm
         if (lim >= user_limit) break;
     }
     for (int q = 0; q < nb; ++q) {
-        if (mode[q] == 3) CU(c, solve_tiled(args[q], c->dtype, c->pool[q], &c->launches));
+        if (mode[q] == 3) {
+            KernelTimeout to;
+            args[q].timeout = &to;
+            rc = solve_status(c, "tiled engine", solve_tiled(args[q], c->dtype, c->pool[q], &c->launches), to);
+            if (rc) return rc;
+        }
         CU(c, cudaEventRecord(c->pool_ev[q], c->pool[q]));
         CU(c, cudaStreamWaitEvent(c->stream, c->pool_ev[q], 0));
     }

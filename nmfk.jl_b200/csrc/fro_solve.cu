@@ -231,7 +231,10 @@ cudaError_t solve_fro_t(const SolveArgs& a, const void* Xlo, const void* Xtlo, c
     T *Ht = nullptr, *Nbuf = nullptr;
     float *Wlo = nullptr, *Htlo = nullptr;
     double *Gpart = nullptr, *convW = nullptr, *convH = nullptr, *objp = nullptr;
-    int *d_active = nullptr, *h_active = nullptr, *d_err = nullptr;
+    int *d_active = nullptr, *h_active = nullptr;
+    int* errflag = nullptr;  // h_active + 1: barrier time-out site, written by the tcgen05 kernels through mapped pinned memory
+    const char* flag_kernel = "fro_gemm_kernel";  // what can raise it in the current phase of the solve, for the error message
+    const char* flag_where = "stacked GEMM of an iteration";
     const int nblkObj = (n + 127) / 128;
     std::vector<UnitState> hst((size_t)R);
     bool any_running = false;
@@ -250,11 +253,11 @@ cudaError_t solve_fro_t(const SolveArgs& a, const void* Xlo, const void* Xtlo, c
     FRO_TRY(scratch_alloc(&convW, (size_t)R * tilesW * k * 2 * sizeof(double), s));
     FRO_TRY(scratch_alloc(&convH, (size_t)R * tilesH * k * 2 * sizeof(double), s));
     FRO_TRY(scratch_alloc(&objp, (size_t)R * nblkObj * 2 * sizeof(double), s));
-    FRO_TRY(scratch_alloc(&d_active, 2 * sizeof(int), s));
-    d_err = d_active + 1;
-    FRO_TRY(cudaMemsetAsync(d_active, 0, 2 * sizeof(int), s));
+    FRO_TRY(scratch_alloc(&d_active, sizeof(int), s));
     h_active = pinned_flags();
     if (h_active == nullptr) FRO_TRY(cudaErrorMemoryAllocation);
+    h_active[0] = h_active[1] = 0;
+    errflag = h_active + 1;
     FRO_TRY(cudaMemcpyAsync(hst.data(), a.st, (size_t)R * sizeof(UnitState), cudaMemcpyDeviceToHost, s));
     FRO_TRY(cudaStreamSynchronize(s));
     for (auto& u : hst)
@@ -283,12 +286,13 @@ cudaError_t solve_fro_t(const SolveArgs& a, const void* Xlo, const void* Xtlo, c
                 tiled_guard_kernel<<<(R + 127) / 128, 128, 0, s>>>(a.st, R, it, a.maxiter, INT_MAX, INT_MAX, a.iter_limit, d_active);
                 FRO_TRY(cudaGetLastError());
                 ++*launches;
-                FRO_TRY(cudaMemcpyAsync(h_active, d_active, 2 * sizeof(int), cudaMemcpyDeviceToHost, s));
+                FRO_TRY(cudaMemcpyAsync(h_active, d_active, sizeof(int), cudaMemcpyDeviceToHost, s));
                 pt.mark(s, 10);
                 FRO_TRY(cudaStreamSynchronize(s));
                 if (a.prof) a.prof->harvest();
                 pt.harvest();
-                if (h_active[0] == 0 || h_active[1] != 0) break;
+                if (h_active[1] != 0) goto done;
+                if (h_active[0] == 0) break;
                 need_guard = false;
                 pt.mark(s, -1);
             }
@@ -300,7 +304,7 @@ cudaError_t solve_fro_t(const SolveArgs& a, const void* Xlo, const void* Xtlo, c
                 if (a.prof) a.prof->begin(s);
                 if (F32)
                     FRO_TRY(launch_fro_gemm(reinterpret_cast<const float*>(W), Wlo, n, static_cast<const float*>(a.X),
-                                            static_cast<const float*>(Xlo), n, reinterpret_cast<float*>(Nbuf), m, (int)Rk, m, n, NSH, Rk * m, d_err, s));
+                                            static_cast<const float*>(Xlo), n, reinterpret_cast<float*>(Nbuf), m, (int)Rk, m, n, NSH, Rk * m, errflag, s));
                 else
                     FRO_TRY(launch_fro_gemm_f64(reinterpret_cast<const double*>(W), n, static_cast<const double*>(a.X), n,
                                                 reinterpret_cast<double*>(Nbuf), m, (int)Rk, m, n, s));
@@ -317,7 +321,7 @@ cudaError_t solve_fro_t(const SolveArgs& a, const void* Xlo, const void* Xtlo, c
                 if (a.prof) a.prof->begin(s);
                 if (F32)
                     FRO_TRY(launch_fro_gemm(reinterpret_cast<const float*>(Ht), Htlo, m, static_cast<const float*>(a.Xt),
-                                            static_cast<const float*>(Xtlo), m, reinterpret_cast<float*>(Nbuf), n, (int)Rk, n, m, NSW, Rk * n, d_err, s));
+                                            static_cast<const float*>(Xtlo), m, reinterpret_cast<float*>(Nbuf), n, (int)Rk, n, m, NSW, Rk * n, errflag, s));
                 else
                     FRO_TRY(launch_fro_gemm_f64(reinterpret_cast<const double*>(Ht), m, static_cast<const double*>(a.Xt), m,
                                                 reinterpret_cast<double*>(Nbuf), n, (int)Rk, n, m, s));
@@ -369,7 +373,9 @@ cudaError_t solve_fro_t(const SolveArgs& a, const void* Xlo, const void* Xtlo, c
         if (F32) {
             po.D = a.X;
             if (tc_pass_supported(po)) {
-                FRO_TRY(launch_tc_objective(po, d_err, s));
+                flag_kernel = "tc_pass_kernel";
+                flag_where = "post-run objective";
+                FRO_TRY(launch_tc_objective(po, errflag, s));
                 done_obj = true;
             }
         } else if (k >= 4) {
@@ -394,7 +400,8 @@ cudaError_t solve_fro_t(const SolveArgs& a, const void* Xlo, const void* Xtlo, c
         pt.report(it, 0);
     }
 done:
-    if (h_active && h_active[1] != 0) fprintf(stderr, "[nmfk] fro_gemm_kernel: barrier time-out at site %d (protocol error)\n", h_active[1]);
+    // a time-out ends in a trap: the solve has usually failed with that CUDA error already, the flag says where
+    if (h_active && h_active[1] != 0) err = solve_timeout(a, err, flag_kernel, flag_where, h_active[1]);
     scratch_free(Ht, s);
     scratch_free(Nbuf, s);
     scratch_free(Wlo, s);

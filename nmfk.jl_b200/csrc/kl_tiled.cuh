@@ -802,6 +802,9 @@ cudaError_t solve_tiled_t(const SolveArgs& a, cudaStream_t s, int64_t* launches)
     int* fin_flag = nullptr;    //              ... and which restarts tiled_scaleW_kernel has to scale
     void* vimg = nullptr;       // tcgen05 pass (k <= 16): V operand images, rebuilt before every half-update
     int* h_active = nullptr;  // [0] running restarts, [1] barrier time-out site reported by the tcgen05 kernel
+    // the tcgen05 kernels that can raise h_active[1] in the current phase of the solve, for the error message
+    const char* flag_kernel = use_tc && tc2_pass_enabled(k) ? "tc2_pass_kernel or tc_pass_kernel" : "tc_pass_kernel";
+    const char* flag_where = "half-update pass or stop-check objective";
     std::vector<UnitState> hst((size_t)R);
     int it = 0;
     bool any_running = false;
@@ -946,6 +949,7 @@ cudaError_t solve_tiled_t(const SolveArgs& a, cudaStream_t s, int64_t* launches)
                 NMFK_TRY(cudaStreamSynchronize(s));
                 if (a.prof) a.prof->harvest();
                 pt.harvest();
+                if (h_active[1] != 0) goto done;  // written by the tcgen05 kernels through the mapped pinned flags
                 if (*h_active == 0) break;
                 need_guard = false;
                 pt.mark(s, -1);
@@ -1057,6 +1061,8 @@ cudaError_t solve_tiled_t(const SolveArgs& a, cudaStream_t s, int64_t* launches)
     {
         // post-run objective on the restored X + normalisation for restarts that stopped in this call
         pt.mark(s, -1);
+        flag_kernel = "tc_pass_kernel";
+        flag_where = "post-run objective";
         if (use_tc && !wobj) {
             NMFK_TRY(launch_tc_objective(obj_args(1, 1), h_active + 1, s));
         } else if (use_td && !wobj) {
@@ -1095,8 +1101,8 @@ cudaError_t solve_tiled_t(const SolveArgs& a, cudaStream_t s, int64_t* launches)
         pt.report(it, sharded ? sh->rank : 0);
     }
 done:
-    if (h_active && h_active[1] != 0)
-        fprintf(stderr, "[nmfk] tc_pass_kernel: barrier time-out at site %d (protocol error)\n", h_active[1]);
+    // a time-out ends in a trap: the solve has usually failed with that CUDA error already, the flag says where
+    if (h_active && h_active[1] != 0) err = solve_timeout(a, err, flag_kernel, flag_where, h_active[1]);
     scratch_free(den, s);
     scratch_free(partial, s);
     scratch_free(objp, s);

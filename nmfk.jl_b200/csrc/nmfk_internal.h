@@ -101,6 +101,15 @@ struct PassProfile {
     }
 };
 
+// A bounded barrier wait of a tcgen05 kernel (tc_ptx.cuh) that timed out during a solve.  The wait writes its site to an
+// error flag in mapped pinned host memory, which stays readable after the kernel traps.  The solver then stops, fills this
+// in and fails; the entry point turns it into an error message naming the kernel and the site.
+struct KernelTimeout {
+    const char* kernel = nullptr;  // nullptr: no time-out
+    const char* where = nullptr;   // which launch of the solve
+    int site = 0;                  // the `where` code of the wait that timed out
+};
+
 // Arguments of one batched KL solve (R restarts at one k).
 struct SolveArgs {
     const void* X;    // n x m column-major, zeros -> lambda, NaN kept
@@ -119,7 +128,15 @@ struct SolveArgs {
     int32_t tiled_tc;        // tiled engine, Float32 without NaN: 1 = tcgen05 kernel (kl_tiled_tc.cu), 0 = scalar-FMA kernel
     const ShardComm* shard;  // non-null: n is the LOCAL row count, the tiled engine all-reduces the k x m partials
     PassProfile* prof;       // non-null: time the pass-kernel launches of the tiled engine
+    KernelTimeout* timeout;  // non-null: where the tiled / FRO solver reports a barrier time-out
 };
+
+// records a barrier time-out reported through a kernel's error flag; the solver returns the value of this call (the CUDA
+// error of the trap that follows the time-out, when the solver has already met it)
+inline cudaError_t solve_timeout(const SolveArgs& a, cudaError_t err, const char* kernel, const char* where, int site) {
+    if (a.timeout != nullptr) *a.timeout = KernelTimeout{kernel, where, site};
+    return err != cudaSuccess ? err : cudaErrorLaunchTimeout;
+}
 
 // threads per restart-CTA of the resident engine: 512 (<=128 registers) while u/acc fit, 256 beyond
 __host__ __device__ constexpr int resident_threads(int Ktemplate) { return Ktemplate <= 12 ? 512 : 256; }

@@ -88,6 +88,33 @@ def test_c3_shape_tcgen05_pass_vs_oracle(ctx):
     _fixed_iterations_vs_oracle(ctx, 10000, 10000, 16, 16, 2, 3, np.float32, 1e-4)
 
 
+def test_c3_variant_fro_vs_oracle(ctx, capfd):
+    """C3 through Variant FRO as bench.py runs it (10000 x 10000 Float32 mixture, k = 16, 64 restarts, Philox initial factors):
+    3 iterations of the stacked solve, which runs the cluster-multicast GEMM over 8 M tiles with 6 / 6 split-K slices and the
+    Gram sums in 4 / 4 slices.  Restarts 0 (first tile), 8 (second tile, the second CTA of a cluster), 15 (holds row 255, the
+    last row of a cluster pair) and 63 (last tile) against the Float64 oracle."""
+    n, m, k, R, niter = 10000, 10000, 16, 64, 3
+    X = synth.mixture(n, m, 16, seed=2015, dtype=np.float32)
+    W0, H0 = synth.philox_inits(2015, R, n, k, m, dtype=np.float32)
+    ctx.set_X(X)
+    b = ctx.batch(k, R)
+    b.set_init(W0, H0)
+    ctx.solve([b], nb.default_params(variant=1, maxiter=niter, normalize=0))
+    out = b.get()
+    b.close()
+    assert np.all(out["iters"] == niter) and np.all(out["stop_reason"] == 1)
+    X64 = X.astype(np.float64)
+    del X
+    delta = float(np.sqrt(np.finfo(np.float32).eps))
+    for r in (0, 8, 15, 63):
+        W, H, _ = o.nmf_multupdate_mse(X64, k, Winit=W0[r].astype(np.float64), Hinit=H0[r].astype(np.float64), maxiter=niter, tol=0.0,
+                                       delta=delta)
+        eW, eH = relerr(out["W"][r], W), relerr(out["H"][r], H)
+        assert eW < 1e-4 and eH < 1e-4, (r, eW, eH)
+    err = capfd.readouterr().err
+    assert "barrier time-out" not in err, err[-2000:]
+
+
 @pytest.mark.parametrize("k", [32, 5, 3])
 def test_c4_shape_tiled_pass_vs_oracle(ctx, k):
     """BASELINE C4 (100000 x 2000 Float64): k = 32 and 5 run the DMMA tiled pass, k = 3 the scalar-FMA pass."""
