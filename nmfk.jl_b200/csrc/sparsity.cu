@@ -44,12 +44,14 @@ __device__ __forceinline__ void sp_terms(T x, T e, double beta, int bmode, T& es
 }
 
 // A_est / A_x of one half-update.  D: data with the own index contiguous (element (o,t) at D[o + t*nown]); U: own factor
-// (element (o,b) at U[o*su_o + b*su_a]); V: other factor ((t,b) at V[t*sv_t + b*sv_a]); outputs [R][nown][KMAX]
+// (element (o,b) at U[o*su_o + b*su_a]); V: other factor ((t,b) at V[t*sv_t + b*sv_a]); outputs [R][nown][KMAX].
+// D is the preprocessed image of X, whose zeros nmfk_set_X replaced by xsub; NMFsparsity never substitutes them (its
+// NMFpreprocessing! call is commented out), so x == xsub counts as 0 here and in sp_objective_kernel
 template <typename T, int KMAX>
 __global__ void __launch_bounds__(SP_T) sp_pass_kernel(const T* __restrict__ D, const T* __restrict__ Ust, const T* __restrict__ Vst,
                                                        long long u_rstride, long long v_rstride, long long su_o, long long su_a,
-                                                       long long sv_t, long long sv_a, int nown, int nred, int k, double lambda,
-                                                       double beta, int bmode, const UnitState* st, T* __restrict__ Aest,
+                                                       long long sv_t, long long sv_a, int nown, int nred, int k, T xsub,
+                                                       double lambda, double beta, int bmode, const UnitState* st, T* __restrict__ Aest,
                                                        T* __restrict__ Ax) {
     __shared__ T Vs[SP_TT][KMAX + 1];
     const int r = blockIdx.y, tid = threadIdx.x;
@@ -80,7 +82,8 @@ __global__ void __launch_bounds__(SP_T) sp_pass_kernel(const T* __restrict__ D, 
 #pragma unroll
                 for (int b = 0; b < KMAX; ++b) p = fma(u[b], Vs[tt][b], p);
                 const T e = p > lam ? p : lam;  // max.(W*H, lambda)
-                const T x = D[(long long)o + (long long)(t0 + tt) * nown];
+                T x = D[(long long)o + (long long)(t0 + tt) * nown];
+                if (x == xsub) x = (T)0;
                 T est, xt;
                 sp_terms<T>(x, e, beta, bmode, est, xt);
 #pragma unroll
@@ -187,10 +190,12 @@ __global__ void __launch_bounds__(256) sp_colnorm_kernel(T* __restrict__ Wst, T*
     }
 }
 
-// divergence(X, max(W*H, lambda)) of rows [128 b, 128 b + 128) -> part[(r * nblk + b)]   (:89-98)
+// divergence(X, max(W*H, lambda)) of rows [128 b, 128 b + 128) -> part[(r * nblk + b)]   (:89-98).  With zeros in X (x == xsub
+// counts as 0) the kl divergence is NaN and the is divergence Inf, as in the reference: the relative-change test then never
+// stops the run
 template <typename T, int KMAX>
 __global__ void __launch_bounds__(SP_T) sp_objective_kernel(const T* __restrict__ X, int n, int m, int k, const T* __restrict__ Wst,
-                                                            const T* __restrict__ Hst, double lambda, double beta, int bmode,
+                                                            const T* __restrict__ Hst, T xsub, double lambda, double beta, int bmode,
                                                             const UnitState* st, double* __restrict__ part) {
     __shared__ T Hs[SP_TT][KMAX + 1];
     __shared__ double red[8];
@@ -218,7 +223,8 @@ __global__ void __launch_bounds__(SP_T) sp_objective_kernel(const T* __restrict_
 #pragma unroll
                 for (int b = 0; b < KMAX; ++b) p = fma(w[b], Hs[jj][b], p);
                 const double e = (double)(p > (T)lambda ? p : (T)lambda);
-                const double x = (double)X[(long long)i + (long long)(j0 + jj) * n];
+                const T xs = X[(long long)i + (long long)(j0 + jj) * n];
+                const double x = xs == xsub ? 0.0 : (double)xs;
                 double d;
                 if (bmode == 2)
                     d = (x - e) * (x - e);
@@ -275,8 +281,8 @@ cudaError_t sp_iteration(const SolveArgs& a, double beta, int bmode, double spar
     cudaError_t e;
     if (!a.Hfixed) {  // own = columns of H: D = X^T, U = H (su_o = k, su_a = 1), V = W (sv_t = 1, sv_a = n)
         sp_pass_kernel<T, KMAX><<<dim3((m + SP_T - 1) / SP_T, R), SP_T, 0, s>>>(static_cast<const T*>(a.Xt), H, W, (long long)k * m,
-                                                                               (long long)n * k, k, 1, 1, n, m, n, k, lam, beta, bmode, a.st,
-                                                                               Aest, Ax);
+                                                                               (long long)n * k, k, 1, 1, n, m, n, k, (T)a.lambda, lam, beta,
+                                                                               bmode, a.st, Aest, Ax);
         if ((e = cudaGetLastError()) != cudaSuccess) return e;
         sp_apply_H_kernel<T, KMAX><<<dim3((m + 255) / 256, R), 256, 0, s>>>(H, k, m, Aest, Ax, sparsity, lam, a.st);
         if ((e = cudaGetLastError()) != cudaSuccess) return e;
@@ -284,8 +290,8 @@ cudaError_t sp_iteration(const SolveArgs& a, double beta, int bmode, double spar
     }
     if (!a.Wfixed) {  // own = rows of W: D = X, U = W (su_o = 1, su_a = n), V = H' (sv_t = k, sv_a = 1)
         sp_pass_kernel<T, KMAX><<<dim3((n + SP_T - 1) / SP_T, R), SP_T, 0, s>>>(static_cast<const T*>(a.X), W, H, (long long)n * k,
-                                                                               (long long)k * m, 1, n, k, 1, n, m, k, lam, beta, bmode, a.st,
-                                                                               Aest, Ax);
+                                                                               (long long)k * m, 1, n, k, 1, n, m, k, (T)a.lambda, lam, beta,
+                                                                               bmode, a.st, Aest, Ax);
         if ((e = cudaGetLastError()) != cudaSuccess) return e;
         sp_colstats_kernel<T, KMAX><<<R, 256, 0, s>>>(W, n, k, Aest, Ax, a.st, cst);
         sp_apply_W_kernel<T, KMAX><<<dim3((n + 255) / 256, R), 256, 0, s>>>(W, n, k, Aest, Ax, cst, lam, a.st);
@@ -293,7 +299,8 @@ cudaError_t sp_iteration(const SolveArgs& a, double beta, int bmode, double spar
         if ((e = cudaGetLastError()) != cudaSuccess) return e;
         *launches += 4;
     }
-    sp_objective_kernel<T, KMAX><<<dim3(nblk, R), SP_T, 0, s>>>(static_cast<const T*>(a.X), n, m, k, W, H, lam, beta, bmode, a.st, part);
+    sp_objective_kernel<T, KMAX><<<dim3(nblk, R), SP_T, 0, s>>>(static_cast<const T*>(a.X), n, m, k, W, H, (T)a.lambda, lam, beta, bmode,
+                                                                   a.st, part);
     sp_state_kernel<T><<<R, 256, 0, s>>>(a.st, H, k, m, part, nblk, sparsity, a.tol, it);
     *launches += 2;
     return cudaGetLastError();

@@ -439,14 +439,22 @@ def execute_singlerun_compute(
     clusterWmatrix: bool = False,
     modifymatrices: bool = True,
     weight=1,
+    method: str = "simple",
     info: Optional[dict] = None,
     **kw,
 ):
     """`execute_singlerun_compute(X::AbstractMatrix, nk; method=:simple, ...)`
     src/NMFkExecute.jl:729-807 with scale=false, transpose=false, mixture=:null.
     X is passed by reference (:740) and comes back restored.  Returns (W, H, objvalue) where
-    objvalue = normnan(X - W*H) (:791-792, a NORM) and rows of H sum to one (:800-804)."""
-    W, H, _ = nmf_multiplicative(X, nk, tol=tol, maxiter=maxiter, weight=weight, info=info, **kw)  # :762
+    objvalue = normnan(X - W*H) (:791-792, a NORM) and rows of H sum to one (:800-804).
+    method="sparsity" solves with NMFsparsity(X, nk; maxiter, tol, kw...) (:757-758) instead: kw takes cost_function,
+    beta_divergence, sparsity and lam (its `lambda`); the weight does not reach it."""
+    if method == "sparsity":
+        W, H, _ = nmf_sparsity(X, nk, maxiter=maxiter, tol=tol, info=info, **kw)  # :757-758
+    elif method == "simple":
+        W, H, _ = nmf_multiplicative(X, nk, tol=tol, maxiter=maxiter, weight=weight, info=info, **kw)  # :762
+    else:
+        raise ValueError("method=:%s is not restated here (:simple and :sparsity are)" % method)
     E = X - W @ H  # :791
     objvalue = normnan(E)  # :792
     if modifymatrices:  # :795-805 (mixture == :null)

@@ -242,3 +242,29 @@ def test_nmfsparsity_oracle_properties():
     inf = {}
     o.nmf_sparsity(X, 3, Winit=W0, Hinit=H0, sparsity=0.1, maxiter=100000, tol=1e-6, info=inf)
     assert inf["stop_reason"] == "tol" and 1 < inf["iters"] < 100000
+
+
+def test_execute_run_sparsity_composes_nmfsparsity_and_normalisation():
+    """execute_run(...; method=:sparsity) reaches NMFsparsity through execute_singlerun_compute (NMFkExecute.jl:757-758): every
+    restart equals nmf_sparsity followed by objvalue = normnan(X - W*H) (:791-792) and the H-row normalisation (:800-804), and
+    the kw (cost_function, sparsity, lam) reach the solver."""
+    rng = np.random.default_rng(12)
+    X = np.asfortranarray(rng.random((25, 3)) @ rng.random((3, 12)) + 0.01)
+    inits = [(rng.random((25, 3)), rng.random((3, 12))) for _ in range(4)]
+    kw = dict(cost_function="kl", sparsity=0.2, lam=1e-8, maxiter=1000, tol=1e-6)
+    det = {}
+    Wa, Ha, phi, rob, aic = o.execute_run(X.copy(), 3, 4, inits=inits, method="sparsity", details=det, **kw)
+    objs = []
+    for i, (W0, H0) in enumerate(inits):
+        inf = {}
+        W, H, _ = o.nmf_sparsity(X.copy(), 3, Winit=W0, Hinit=H0, info=inf, **kw)
+        objs.append(o.normnan(X - W @ H))
+        total = H.sum(axis=1, keepdims=True)
+        assert np.array_equal(det["WBig"][i], W * total.T) and np.array_equal(det["HBig"][i], H / total), i
+        assert det["iters"][i] == inf["iters"] and det["stop_reasons"][i] == inf["stop_reason"], i
+    assert np.array_equal(det["objvalue"], objs) and np.array_equal(det["idxsort"], np.argsort(objs, kind="stable"))
+    assert set(det["stop_reasons"]) == {"tol"}  # tol reached: the keyword arrived
+    _, _, objd = o.execute_singlerun_compute(X.copy(), 3, Winit=inits[0][0], Hinit=inits[0][1], maxiter=1000, tol=1e-6)
+    assert objd != objs[0]  # method=:simple solves another problem
+    with pytest.raises(ValueError):
+        o.execute_singlerun_compute(X.copy(), 3, method="nmf", Winit=inits[0][0], Hinit=inits[0][1])
