@@ -413,7 +413,10 @@ __global__ void __launch_bounds__((Tc2Cfg<K8>::THREADS), 1) tc2_pass_kernel(cons
                 tc::mbar_wait_h(0u, &p_full[grp], (uint32_t)((u >> 1) & 1), errflag, 41);
                 tc::tc_fence_after_sync();
                 if (warp == QW0) TC_STAMP(0, u, 1);
-#pragma unroll 1
+                // both halves unrolled, so what depends on the half (the p_empty arrive, the a_full wait, the numerator drain,
+                // the column offsets) is fixed at compile time: 96 registers, 0 spills, and 10 % less time per launch on C3
+                // than the rolled loop (DESIGN.md 4a)
+#pragma unroll
                 for (int half = 0; half < 2; ++half) {
                     uint32_t p[16];
                     tc::tmem_ld16(pcol + half * 16, p);
