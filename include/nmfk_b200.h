@@ -92,7 +92,8 @@ typedef struct nmfk_params {
     int32_t stop_rule;      /* 0 = NMFmultiplicative(::AbstractMatrix) (NMFkMultiplicative.jl:64-118);
                                1 = NMFmultiplicative(::DArray) (:129-197): no tolOF/baditers/reattempts logic, no weight,
                                    no NaN imputation; stops on objvalue < tol, inc > stopconv (default 10000) or maxiter */
-    int32_t variant;        /* nmfk_variant: 0 = KL (method=:simple), 1 = FRO (method=:nmf, algorithm=:multdiv) */
+    int32_t variant;        /* nmfk_variant: 0 = KL (method=:simple), 1 = FRO (method=:nmf, algorithm=:multdiv),
+                               2 = SPARSITY (method=:sparsity), 3 = KL_DIV (method=:nmf, algorithm=:multmse) */
     int32_t reserved[1];
 } nmfk_params;
 
@@ -105,8 +106,16 @@ typedef struct nmfk_params {
  *   with the 3-term split for Float32, DMMA for Float64).  Stops when every column of W and row of H moved by less than
  *   `tol` relative (NMF.jl stop_condition) or at maxiter.
  * NMFK_VARIANT_SPARSITY : NMFsparsity (NMFkSparsity.jl:1-113; method=:sparsity, NMFkExecute.jl:757-758): beta-divergence updates
- *   with an L1 penalty on H and unit-norm columns of W; its own options come from nmfk_set_sparsity_options. */
-enum nmfk_variant { NMFK_VARIANT_KL = 0, NMFK_VARIANT_FRO = 1, NMFK_VARIANT_SPARSITY = 2 };
+ *   with an L1 penalty on H and unit-norm columns of W; its own options come from nmfk_set_sparsity_options.
+ * NMFK_VARIANT_KL_DIV : Q = X ./ (W*H .+ d), H .*= (W'Q) ./ (colsum(W)' .+ d), then the same with the new H for
+ *   W .*= (Q*H') ./ (rowsum(H)' .+ d), d = sqrt(eps(T)): the update execute_singlerun_compute reaches with method=:nmf,
+ *   algorithm=:multmse (NMFkExecute.jl:765-768: NMF.MultUpdate(obj=:div), third-party NMF.jl, restated in
+ *   tests/test_oracle_multmse_cpu.py).  The KL update of method=:simple with d added, on the tiled engine's passes for every size and
+ *   engine choice (tcgen05 for Float32, DMMA for Float64 with k >= 4, scalar FMA otherwise; k <= 64); no lambda imputation,
+ *   clamp or objective checks.  Stops when every column of W and row of H moved by less than `tol` relative (NMF.jl
+ *   stop_condition, checked after every iteration) or at maxiter.  Not available with NaN in X, a row-sharded ctx,
+ *   normalizevector, array weights, stop_rule 1 or the resident engines. */
+enum nmfk_variant { NMFK_VARIANT_KL = 0, NMFK_VARIANT_FRO = 1, NMFK_VARIANT_SPARSITY = 2, NMFK_VARIANT_KL_DIV = 3 };
 
 /* Solution filtering of execute_run (NMFkExecute.jl:551-596): which of the R sorted restarts reach clustersolutions /
  * finalize.  Defaults acceptratio=1, acceptfactor=Inf, nanaction=:zeroed keep all of them. */

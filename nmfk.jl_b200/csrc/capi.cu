@@ -688,7 +688,7 @@ static int32_t check_params(nmfk_ctx* c, const nmfk_params* p) {
         return fail(c, NMFK_E_INVALID, "params: check_every, maxbaditers, maxreattempts must be >= 1, maxiter >= 0");
     if (p->normalize < 0 || p->normalize > 2) return fail(c, NMFK_E_INVALID, "params: normalize must be 0, 1 or 2");
     if (p->stop_rule < 0 || p->stop_rule > 1) return fail(c, NMFK_E_INVALID, "params: stop_rule must be 0 or 1");
-    if (p->variant < NMFK_VARIANT_KL || p->variant > NMFK_VARIANT_SPARSITY) return fail(c, NMFK_E_INVALID, "params: unknown variant");
+    if (p->variant < NMFK_VARIANT_KL || p->variant > NMFK_VARIANT_KL_DIV) return fail(c, NMFK_E_INVALID, "params: unknown variant");
     if (p->stop_rule == 1 && c && c->info.nnan > 0)
         return fail(c, NMFK_E_UNSUPPORTED, "stop_rule 1 (the DArray method) with NaN entries in X is not supported: the reference "
                                            "itself returns objvalue = NaN there (NMFkMultiplicative.jl:193-195)");
@@ -742,7 +742,7 @@ static void fill_args(const nmfk_batch* b, const nmfk_params* p, SolveArgs& a) {
 
 // tiled engine (kl_tiled.cu): host-driven, for factors that do not fit in shared memory
 namespace nmfk {
-cudaError_t solve_tiled(const SolveArgs& a, int dtype, cudaStream_t s, int64_t* launches);
+cudaError_t solve_tiled(const SolveArgs& a, int dtype, cudaStream_t s, int64_t* launches, bool div = false);
 bool tiled_supported(int k);
 }  // namespace nmfk
 
@@ -845,6 +845,35 @@ static int32_t solve_sparsity_batches(nmfk_ctx* c, nmfk_batch* const* batches, i
     return NMFK_OK;
 }
 
+// Variant KL_DIV (method=:nmf, algorithm=:multmse; NMFkExecute.jl:765-768): the tiled engine's passes in their delta flavour,
+// one batch after the other.  Every size runs on the tiled engine (there is no resident flavour).
+static int32_t solve_kl_div_batches(nmfk_ctx* c, nmfk_batch* const* batches, int32_t nb, const nmfk_params* p) {
+    if (c->info.nnan > 0) return fail(c, NMFK_E_UNSUPPORTED, "variant KL_DIV: X holds NaN (NMF.jl's MultUpdate has no missing-data handling)");
+    if (c->sharded) return fail(c, NMFK_E_UNSUPPORTED, "variant KL_DIV: row-sharded X is not available");
+    if (c->Xn) return fail(c, NMFK_E_UNSUPPORTED, "variant KL_DIV: normalizevector is not available");
+    if (c->wrow || c->wcol || c->wmat) return fail(c, NMFK_E_UNSUPPORTED, "variant KL_DIV: array weights are not available");
+    if (p->stop_rule != 0) return fail(c, NMFK_E_UNSUPPORTED, "variant KL_DIV has its own stop rule (NMF.jl stop_condition)");
+    if (p->engine == NMFK_ENGINE_RESIDENT || p->engine == NMFK_ENGINE_RESIDENT_SCALAR)
+        return fail(c, NMFK_E_UNSUPPORTED, "variant KL_DIV: only the tiled engine is available");
+    for (int i = 0; i < nb; ++i)
+        if (!tiled_supported(batches[i]->k)) return fail(c, NMFK_E_UNSUPPORTED, "variant KL_DIV: k > 64 is not supported");
+    CU(c, cudaEventRecord(c->ev0, c->stream));
+    for (int i = 0; i < nb; ++i) {
+        SolveArgs a;
+        fill_args(batches[i], p, a);
+        KernelTimeout to;
+        a.timeout = &to;
+        const int32_t rc = solve_status(c, "variant KL_DIV", solve_tiled(a, c->dtype, c->stream, &c->launches, true), to);
+        if (rc) return rc;
+    }
+    CU(c, cudaEventRecord(c->ev1, c->stream));
+    CU(c, cudaEventSynchronize(c->ev1));
+    float ms = 0.f;
+    CU(c, cudaEventElapsedTime(&ms, c->ev0, c->ev1));
+    c->last_solve_ms = ms;
+    return NMFK_OK;
+}
+
 int32_t nmfk_set_sparsity_options(nmfk_ctx* c, double beta_divergence, double sparsity, double lambda) {
     if (!c) return fail(nullptr, NMFK_E_INVALID, "ctx is NULL");
     if (!(lambda > 0)) return fail(c, NMFK_E_INVALID, "nmfk_set_sparsity_options: lambda must be positive");
@@ -866,6 +895,7 @@ int32_t nmfk_solve(nmfk_ctx* c, nmfk_batch* const* batches, int32_t nb, const nm
     }
     if (p->variant == NMFK_VARIANT_FRO) return solve_fro_batches(c, batches, nb, p);
     if (p->variant == NMFK_VARIANT_SPARSITY) return solve_sparsity_batches(c, batches, nb, p);
+    if (p->variant == NMFK_VARIANT_KL_DIV) return solve_kl_div_batches(c, batches, nb, p);
     while ((int)c->pool.size() < nb) {
         cudaStream_t s;
         cudaEvent_t ev;

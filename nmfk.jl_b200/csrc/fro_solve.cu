@@ -422,6 +422,12 @@ cudaError_t launch_sum_slices(float* C, int S, long long pstride, long long len,
     return cudaGetLastError();
 }
 
+cudaError_t launch_fro_converge(UnitState* st, int R, int k, const double* convW, int tilesW, const double* convH, int tilesH,
+                                int wactive, int hactive, double tol, int it, cudaStream_t s) {
+    fro_converge_kernel<<<(R + 127) / 128, 128, 0, s>>>(st, R, k, convW, tilesW, convH, tilesH, wactive, hactive, tol, it);
+    return cudaGetLastError();
+}
+
 cudaError_t launch_split_lo(const float* x, float* lo, long long len, cudaStream_t s) {
     split_lo_kernel<<<148 * 8, 256, 0, s>>>(x, lo, len);
     return cudaGetLastError();

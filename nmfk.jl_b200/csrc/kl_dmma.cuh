@@ -221,7 +221,8 @@ __device__ __forceinline__ int dmma_sigma(int c) { return c < 4 ? c : (c ^ 1); }
 // MODE 0: fast reciprocal, no range check (the caller tests the accumulators for NaN and redoes the item);
 // MODE 1: IEEE divisions, steps beyond the end masked; MODE 2: fast reciprocal with a warp-uniform range
 // check that falls back to IEEE divisions (tiled engine: an item cannot be redone once its V chunks are gone).
-template <int K, int MODE, int NT, int SET0>
+// DIV: the quotient of NMF.jl's KL update (Variant KL_DIV), x / (p + kKlDivDelta).
+template <int K, int MODE, int NT, int SET0, bool DIV = false>
 __device__ __forceinline__ void dmma_tiles(DmmaRegs<K>& R, const double (&x)[NT][2], const double* __restrict__ vp1,
                                            const double* __restrict__ vp2a, const double* __restrict__ vp2b, int g,
                                            const bool (&in)[NT][2], bool hi_ok) {
@@ -260,6 +261,13 @@ __device__ __forceinline__ void dmma_tiles(DmmaRegs<K>& R, const double (&x)[NT]
     for (int kc = 0; kc < C::KCD; ++kc)
 #pragma unroll
         for (int j = 0; j < NT; ++j) dmma884(p[j], R.ua[kc], vp1[j * TS + kc * 4]);
+    if constexpr (DIV) {
+#pragma unroll
+        for (int j = 0; j < NT; ++j) {
+            p[j][0] += kKlDivDelta<double>;
+            p[j][1] += kKlDivDelta<double>;
+        }
+    }
 #pragma unroll
     for (int j = 0; j < NT; ++j) {
         if constexpr (MODE == 1) {

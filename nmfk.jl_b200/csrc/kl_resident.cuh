@@ -160,7 +160,8 @@ __device__ __forceinline__ TC dot2(const TC (&u)[KP], const TC (&v)[KP]) {
 // divisions, then K independent accumulator chains (acc[a] += V[t][a] * x_t / (u . V[t,:])).
 // V rows are re-read from shared memory for the accumulation phase instead of being kept live
 // (registers are the scarce resource: u and acc already hold 2K values).
-template <typename TC, int K, int KP, int UNR>
+// DIV: the quotient of NMF.jl's KL update (Variant KL_DIV), x / (u . V[t,:] + kKlDivDelta).
+template <typename TC, int K, int KP, int UNR, bool DIV = false>
 __device__ __forceinline__ void kl_group(const TC (&x)[UNR], const TC* const (&vrow)[UNR], const bool (&live)[UNR],
                                          const TC (&u)[KP], TC (&acc)[KP]) {
     TC p[UNR], qv[UNR];
@@ -170,6 +171,7 @@ __device__ __forceinline__ void kl_group(const TC (&x)[UNR], const TC* const (&v
         TC v[KP];
         load_row<TC, KP>(vrow[q], v);
         p[q] = dot2<TC, K, KP>(u, v);
+        if constexpr (DIV) p[q] += kKlDivDelta<TC>;
     }
 #pragma unroll
     for (int q = 0; q < UNR; ++q) {

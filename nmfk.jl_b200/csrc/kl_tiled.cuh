@@ -41,7 +41,9 @@ struct TiledCfg {
 };
 
 
-template <typename TX, typename TC, int K, bool HASNAN>
+// DIV (HASNAN = false only): the quotient of NMF.jl's KL update (Variant KL_DIV), x / (p + delta); a.den already holds the sums
+// + delta
+template <typename TX, typename TC, int K, bool HASNAN, bool DIV = false>
 __global__ void __launch_bounds__(kTiledThreads, (K <= 12 ? 2 : 1)) tiled_pass_kernel(const TiledPassArgs a) {
     constexpr int VEC = VecOf<TC>::N;
     constexpr int KP = (K + VEC - 1) / VEC * VEC;
@@ -148,7 +150,7 @@ __global__ void __launch_bounds__(kTiledThreads, (K <= 12 ? 2 : 1)) tiled_pass_k
                     }
                     vrow[q] = vs + tq * KP;
                 }
-                kl_group<TC, K, KP, UNR>(x, vrow, live, u, acc);
+                kl_group<TC, K, KP, UNR, DIV>(x, vrow, live, u, acc);
             }
         }
     }
@@ -538,6 +540,43 @@ __global__ void __launch_bounds__(256) tiled_finish_kernel(void* Wv, void* Hv, U
     if (tid == 0) st->done = 1;
 }
 
+// Variant KL_DIV: den[r][a] += delta (NMF.jl's colsum(W) .+ delta / rowsum(H) .+ delta) for every running restart
+template <typename TC>
+__global__ void tiled_den_delta_kernel(TC* __restrict__ den, int k, const UnitState* st) {
+    const int r = blockIdx.x, c = threadIdx.x;
+    if (st[r].stop != 0 || c >= k) return;
+    den[(long long)r * kTiledMaxK + c] += kKlDivDelta<TC>;
+}
+
+// Variant KL_DIV: the sums of NMF.jl's stop_condition for one factor against its snapshot from before the iteration, in the
+// layout fro_converge_kernel reads: conv[((r * gridDim.x + tile) * k + a) * 2 + {0,1}] = sum over the tile's 256 own indices o of
+// (new - old)^2, (new + old)^2 for column a of W (o = row) or row a of H (o = column).
+template <typename TC>
+__global__ void __launch_bounds__(256) tiled_conv_kernel(const TC* __restrict__ U, const TC* __restrict__ Uold, long long rstride,
+                                                          long long s_o, long long s_a, int nown, int k, const UnitState* st,
+                                                          double* __restrict__ conv) {
+    __shared__ double red[40];
+    const int r = blockIdx.y, tile = blockIdx.x;
+    if (st[r].stop != 0) return;
+    const int o = tile * 256 + threadIdx.x;
+    const long long base = (long long)r * rstride + (long long)o * s_o;
+    for (int c = 0; c < k; ++c) {
+        double d2 = 0.0, s2 = 0.0;
+        if (o < nown) {
+            const double un = (double)U[base + (long long)c * s_a], uo = (double)Uold[base + (long long)c * s_a];
+            d2 = (un - uo) * (un - uo);
+            s2 = (un + uo) * (un + uo);
+        }
+        d2 = block_sum(d2, red);
+        s2 = block_sum(s2, red);
+        if (threadIdx.x == 0) {
+            double* dst = conv + (((long long)r * gridDim.x + tile) * k + c) * 2;
+            dst[0] = d2;
+            dst[1] = s2;
+        }
+    }
+}
+
 // loop guard of :64 evaluated on the device between iterations: marks restarts that must not start
 // another iteration and counts the ones still running
 static __global__ void tiled_guard_kernel(UnitState* st, int R, int it, int maxiter, int maxbad, int maxre, int iter_limit,
@@ -560,7 +599,7 @@ static __global__ void tiled_guard_kernel(UnitState* st, int R, int it, int maxi
 // red == nullptr: the complete half-update.  red != nullptr (row-sharded X, H-update): the pass leaves
 // the numerators of this rank's rows in red[R][nown][K]; launch_tiled_apply_k finishes after the all-reduce.
 template <typename TX, typename TC, int K>
-cudaError_t launch_tiled_pass_k(const TiledPassArgs& a, void* red, cudaStream_t s) {
+cudaError_t launch_tiled_pass_k(const TiledPassArgs& a, void* red, cudaStream_t s, bool div = false) {
     constexpr int VEC = VecOf<TC>::N;
     constexpr int KP = (K + VEC - 1) / VEC * VEC;
     constexpr int TCH = TiledCfg<TX>::TCH;
@@ -568,7 +607,11 @@ cudaError_t launch_tiled_pass_k(const TiledPassArgs& a, void* red, cudaStream_t 
     const long long grid = (long long)a.S * a.nblocks * a.R;
     if (grid > 2147483647ll) return cudaErrorInvalidValue;
     cudaError_t e;
-    if (a.has_nan) {
+    if (div) {
+        e = cudaFuncSetAttribute(tiled_pass_kernel<TX, TC, K, false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+        if (e != cudaSuccess) return e;
+        tiled_pass_kernel<TX, TC, K, false, true><<<(unsigned)grid, kTiledThreads, smem, s>>>(a);
+    } else if (a.has_nan) {
         e = cudaFuncSetAttribute(tiled_pass_kernel<TX, TC, K, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
         if (e != cudaSuccess) return e;
         tiled_pass_kernel<TX, TC, K, true><<<(unsigned)grid, kTiledThreads, smem, s>>>(a);
@@ -642,28 +685,30 @@ cudaError_t dispatch_tiled_combine(const TiledPassArgs& a, void* red, cudaStream
 // use_tc: Float32 without NaN -> the tcgen05 kernel of kl_tiled_tc.cu (a.nblocks counts 128-index tiles)
 // use_td: Float64 without NaN, k >= 4 -> the DMMA kernel of kl_tiled_dmma.cu (a.nblocks counts 128-index blocks, a.D is
 // the step-contiguous copy of the data)
+// div: the pass kernels' Variant KL_DIV flavour (quotient x / (p + delta); a.den holds the sums + delta)
 template <typename TX, typename TC>
-cudaError_t dispatch_tiled_pass(const TiledPassArgs& a, void* red, cudaStream_t s, bool use_tc, int* errflag, bool use_td = false) {
+cudaError_t dispatch_tiled_pass(const TiledPassArgs& a, void* red, cudaStream_t s, bool use_tc, int* errflag, bool use_td = false,
+                                bool div = false) {
     const int kt = tiled_template_k(a.k);
     if (use_tc) {
-        cudaError_t e = launch_tc_pass(a, errflag, s);
+        cudaError_t e = launch_tc_pass(a, errflag, s, div);
         if (e != cudaSuccess || a.partial == nullptr) return e;
         return dispatch_tiled_combine<TX, TC>(a, red, s);
     }
     if (use_td) {
-        cudaError_t e = launch_tiled_dmma_pass(a, s);
+        cudaError_t e = launch_tiled_dmma_pass(a, s, div);
         if (e != cudaSuccess || a.partial == nullptr) return e;
         return dispatch_tiled_combine<TX, TC>(a, red, s);
     }
-    NMFK_DISPATCH_TILED_K(launch_tiled_pass_k, TX, TC, kt, a, red, s)
+    NMFK_DISPATCH_TILED_K(launch_tiled_pass_k, TX, TC, kt, a, red, s, div)
 }
 // the same, bracketed by the profile events (one "launch" = the pass kernel, plus the small slice-combine kernel when the
 // reduction range is sliced)
 template <typename TX, typename TC>
 cudaError_t timed_tiled_pass(const TiledPassArgs& a, void* red, cudaStream_t s, bool use_tc, int* errflag, bool use_td,
-                             PassProfile* prof) {
+                             PassProfile* prof, bool div = false) {
     if (prof) prof->begin(s);
-    const cudaError_t e = dispatch_tiled_pass<TX, TC>(a, red, s, use_tc, errflag, use_td);
+    const cudaError_t e = dispatch_tiled_pass<TX, TC>(a, red, s, use_tc, errflag, use_td, div);
     if (prof) prof->end(s);
     return e;
 }
@@ -676,7 +721,7 @@ cudaError_t dispatch_tiled_apply(const TiledPassArgs& a, void* red, cudaStream_t
 // NMFK_TILED_TIMING=1: device time of every phase of the tiled engine's iteration (CUDA events between the launches, read at
 // the host synchronisation points), printed per solve - the timeline that says what bounds an iteration (row-sharded runs).
 struct PhaseTimer {
-    static constexpr int NPH = 12;
+    static constexpr int NPH = 14;
     bool on = false;
     std::vector<cudaEvent_t> idle;
     std::vector<std::pair<cudaEvent_t, int>> marks;
@@ -708,7 +753,7 @@ struct PhaseTimer {
     void report(int iters, int rank) {
         if (!on) return;
         static const char* names[NPH] = {"sums_W", "pass_H", "allreduce_H", "apply_H", "sums_H", "pass_W", "impute", "objective",
-                                         "objsum_allreduce", "clamp_check", "guard_sync", "finish"};
+                                         "objsum_allreduce", "clamp_check", "guard_sync", "finish", "snapshot", "converge"};
         fprintf(stderr, "[nmfk timing rank %d] %d iterations:", rank, iters);
         for (int i = 0; i < NPH; ++i)
             if (cnt[i]) fprintf(stderr, " %s=%.3fms/%lld", names[i], ms[i], cnt[i]);
@@ -727,11 +772,15 @@ struct PhaseTimer {
         }                                   \
     } while (0)
 
+// div: Variant KL_DIV (NMF.jl's MultUpdate(obj=:div)) instead of NMFmultiplicative: the same passes in their delta flavour,
+// no NaN imputation, clamp or objective checks; NMF.jl's stop_condition after every iteration against a snapshot of the factors
+// taken before it (fro_converge_kernel), the host looking at the running count every check_every iterations
 template <typename TX, typename TC>
-cudaError_t solve_tiled_t(const SolveArgs& a, cudaStream_t s, int64_t* launches) {
+cudaError_t solve_tiled_t(const SolveArgs& a, cudaStream_t s, int64_t* launches, bool div) {
     const int n = a.n, m = a.m, k = a.k, R = a.R;
     const int kt = tiled_template_k(k);
     if (kt < 0) return cudaErrorInvalidValue;
+    if (div && (a.has_nan || a.shard != nullptr)) return cudaErrorNotSupported;
     cudaError_t err = cudaSuccess;
     int sms = 148;
     {
@@ -800,6 +849,11 @@ cudaError_t solve_tiled_t(const SolveArgs& a, cudaStream_t s, int64_t* launches)
     int* d_active = nullptr;
     double* fin_tot = nullptr;  // wide finish: the k totals of every restart
     int* fin_flag = nullptr;    //              ... and which restarts tiled_scaleW_kernel has to scale
+    TC* Wold = nullptr;         // Variant KL_DIV: the factors before the iteration ...
+    TC* Hold = nullptr;
+    double* convW = nullptr;    // ... and the per-tile sums of the stop condition
+    double* convH = nullptr;
+    const int ctW = (n + 255) / 256, ctH = (m + 255) / 256;
     void* vimg = nullptr;       // tcgen05 pass (k <= 16): V operand images, rebuilt before every half-update
     int* h_active = nullptr;  // [0] running restarts, [1] barrier time-out site reported by the tcgen05 kernel
     // the tcgen05 kernels that can raise h_active[1] in the current phase of the solve, for the error message
@@ -856,6 +910,12 @@ cudaError_t solve_tiled_t(const SolveArgs& a, cudaStream_t s, int64_t* launches)
     NMFK_TRY(scratch_alloc(&d_active, sizeof(int), s));
     NMFK_TRY(scratch_alloc(&fin_tot, (size_t)R * kTiledMaxK * sizeof(double), s));
     NMFK_TRY(scratch_alloc(&fin_flag, (size_t)R * sizeof(int), s));
+    if (div) {
+        NMFK_TRY(scratch_alloc(&Wold, (size_t)R * n * k * sizeof(TC), s));
+        NMFK_TRY(scratch_alloc(&Hold, (size_t)R * k * m * sizeof(TC), s));
+        NMFK_TRY(scratch_alloc(&convW, (size_t)R * ctW * k * 2 * sizeof(double), s));
+        NMFK_TRY(scratch_alloc(&convH, (size_t)R * ctH * k * 2 * sizeof(double), s));
+    }
     if (use_tc) {
         const size_t vb = std::max(tc2_image_bytes(k, R, n), tc2_image_bytes(k, R, m));
         if (vb) NMFK_TRY(scratch_alloc(&vimg, vb, s));
@@ -940,8 +1000,8 @@ cudaError_t solve_tiled_t(const SolveArgs& a, cudaStream_t s, int64_t* launches)
         while (true) {
             if (need_guard) {
                 NMFK_TRY(cudaMemsetAsync(d_active, 0, sizeof(int), s));
-                tiled_guard_kernel<<<(R + 127) / 128, 128, 0, s>>>(a.st, R, it, a.maxiter, a.maxbad, a.maxre, a.iter_limit,
-                                                                   d_active);
+                tiled_guard_kernel<<<(R + 127) / 128, 128, 0, s>>>(a.st, R, it, a.maxiter, div ? INT_MAX : a.maxbad,
+                                                                   div ? INT_MAX : a.maxre, a.iter_limit, d_active);
                 NMFK_TRY(cudaGetLastError());
                 ++*launches;
                 NMFK_TRY(cudaMemcpyAsync(h_active, d_active, sizeof(int), cudaMemcpyDeviceToHost, s));
@@ -956,11 +1016,21 @@ cudaError_t solve_tiled_t(const SolveArgs& a, cudaStream_t s, int64_t* launches)
             }
             ++it;
             ph.first_iter = pw.first_iter = (it == 1);
+            if (div) {
+                if (!a.Wfixed) NMFK_TRY(cudaMemcpyAsync(Wold, a.W, (size_t)R * n * k * sizeof(TC), cudaMemcpyDeviceToDevice, s));
+                if (!a.Hfixed) NMFK_TRY(cudaMemcpyAsync(Hold, a.H, (size_t)R * k * m * sizeof(TC), cudaMemcpyDeviceToDevice, s));
+                pt.mark(s, 12);
+            }
             if (!a.Hfixed) {
                 tiled_sums_kernel<TC><<<dim3(k, R), 256, 0, s>>>(a.W, (long long)n * k, 1, n, n, a.st, den);
                 NMFK_TRY(cudaGetLastError());
+                if (div) {
+                    tiled_den_delta_kernel<TC><<<R, kTiledMaxK, 0, s>>>(den, k, a.st);
+                    NMFK_TRY(cudaGetLastError());
+                    ++*launches;
+                }
                 pt.mark(s, 0);
-                NMFK_TRY((timed_tiled_pass<TX, TC>(ph, red, s, use_tc, h_active + 1, use_td, a.prof)));
+                NMFK_TRY((timed_tiled_pass<TX, TC>(ph, red, s, use_tc, h_active + 1, use_td, a.prof, div)));
                 pt.mark(s, 1);
                 *launches += 2 + (SH > 1 || sharded) + (vimg != nullptr);  // + the image producer of the tc2 pass
                 if (d_trace != nullptr) {
@@ -987,8 +1057,13 @@ cudaError_t solve_tiled_t(const SolveArgs& a, cudaStream_t s, int64_t* launches)
             if (!a.Wfixed) {
                 tiled_sums_kernel<TC><<<dim3(k, R), 256, 0, s>>>(a.H, (long long)k * m, k, 1, m, a.st, den);
                 NMFK_TRY(cudaGetLastError());
+                if (div) {
+                    tiled_den_delta_kernel<TC><<<R, kTiledMaxK, 0, s>>>(den, k, a.st);
+                    NMFK_TRY(cudaGetLastError());
+                    ++*launches;
+                }
                 pt.mark(s, 4);
-                NMFK_TRY((timed_tiled_pass<TX, TC>(pw, nullptr, s, use_tc, h_active + 1, use_td, a.prof)));
+                NMFK_TRY((timed_tiled_pass<TX, TC>(pw, nullptr, s, use_tc, h_active + 1, use_td, a.prof, div)));
                 pt.mark(s, 5);
                 *launches += 2 + (SW > 1) + (vimg != nullptr);
             }
@@ -999,7 +1074,22 @@ cudaError_t solve_tiled_t(const SolveArgs& a, cudaStream_t s, int64_t* launches)
                 NMFK_TRY(cudaGetLastError());
                 ++*launches;
             }
-            if (it % a.check_every == 0) {
+            if (div) {
+                if (!a.Wfixed) {
+                    tiled_conv_kernel<TC><<<dim3(ctW, R), 256, 0, s>>>((const TC*)a.W, Wold, (long long)n * k, 1, n, n, k, a.st, convW);
+                    NMFK_TRY(cudaGetLastError());
+                    ++*launches;
+                }
+                if (!a.Hfixed) {
+                    tiled_conv_kernel<TC><<<dim3(ctH, R), 256, 0, s>>>((const TC*)a.H, Hold, (long long)k * m, k, 1, m, k, a.st, convH);
+                    NMFK_TRY(cudaGetLastError());
+                    ++*launches;
+                }
+                NMFK_TRY(launch_fro_converge(a.st, R, k, convW, ctW, convH, ctH, !a.Wfixed, !a.Hfixed, a.tol, it, s));
+                ++*launches;
+                pt.mark(s, 13);
+                if (it % a.check_every == 0) need_guard = true;
+            } else if (it % a.check_every == 0) {
                 if (use_tc && !wobj) {
                     NMFK_TRY(launch_tc_objective(obj_args(0, 0), h_active + 1, s));
                 } else if (use_td && !wobj) {
@@ -1111,6 +1201,10 @@ done:
     scratch_free(fin_tot, s);
     scratch_free(fin_flag, s);
     scratch_free(vimg, s);
+    scratch_free(Wold, s);
+    scratch_free(Hold, s);
+    scratch_free(convW, s);
+    scratch_free(convH, s);
     return err;
 }
 

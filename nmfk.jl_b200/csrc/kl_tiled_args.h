@@ -39,10 +39,11 @@ bool tc_pass_supported(const TiledPassArgs& a);
 int tc_pass_group(int k);  // restarts that share one X tile inside a CTA
 int tc_pass_ctas_per_sm(int k);
 int tc_pass_chunk(int k);  // steps per chunk (slices hold whole chunks)
-cudaError_t launch_tc_pass(const TiledPassArgs& a, int* d_errflag, cudaStream_t s);
+// div: the quotient flavour of Variant KL_DIV, x / (p + kKlDivDelta) (a.den must already hold the sums + kKlDivDelta)
+cudaError_t launch_tc_pass(const TiledPassArgs& a, int* d_errflag, cudaStream_t s, bool div = false);
 // second generation for k <= 16 (kl_tiled_tc2.cu): U in shared memory, separate P and Q tiles; same grid and arguments
 bool tc2_pass_enabled(int k);
-cudaError_t launch_tc2_pass(const TiledPassArgs& a, int* d_errflag, cudaStream_t s);
+cudaError_t launch_tc2_pass(const TiledPassArgs& a, int* d_errflag, cudaStream_t s, bool div = false);
 // scratch of the tc2 pass (a.vimg): the V operand images of R restarts over a reduction range of nred steps (0: the pass does
 // not serve k).  A launch first builds the images of its running restarts there, then the pass copies them into shared memory.
 size_t tc2_image_bytes(int k, int R, int nred);
@@ -57,7 +58,12 @@ cudaError_t launch_tc_objective(const TiledPassArgs& a, int* d_errflag, cudaStre
 // nblocks = ceil(nown / tiled_dmma_own()), 4 <= k <= 64, no NaN.
 int tiled_dmma_own();
 int tiled_dmma_chunk();
-cudaError_t launch_tiled_dmma_pass(const TiledPassArgs& a, cudaStream_t s);
+cudaError_t launch_tiled_dmma_pass(const TiledPassArgs& a, cudaStream_t s, bool div = false);
 cudaError_t launch_tiled_dmma_objective(const TiledPassArgs& a, cudaStream_t s);
+
+// NMF.jl stop_condition after an iteration (fro_solve.cu's fro_converge_kernel): restarts whose every column of W and row of H
+// moved by less than tol relative stop with reason 2.  convW / convH: per-tile sums, [((r * tiles + tile) * k + a) * 2 + {0,1}]
+cudaError_t launch_fro_converge(UnitState* st, int R, int k, const double* convW, int tilesW, const double* convH, int tilesH,
+                                int wactive, int hactive, double tol, int it, cudaStream_t s);
 
 }  // namespace nmfk

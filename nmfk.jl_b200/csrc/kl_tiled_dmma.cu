@@ -48,7 +48,8 @@ __device__ __forceinline__ void dmma_p_tile(const DmmaRegs<K>& R, const double* 
 
 // OBJ = true: objective mode (NMFkMultiplicative.jl:74,125): only P = U V^T, the lanes accumulate (x - p)^2; nothing is
 // written to the factors.  a = the W-update arguments with S = 1; partial sums per block of 128 rows.
-template <int K, bool OBJ>
+// DIV (pass mode only): the quotient of NMF.jl's KL update (Variant KL_DIV), x / (p + delta); a.den already holds the sums + delta
+template <int K, bool OBJ, bool DIV = false>
 __global__ void __launch_bounds__(TD_THREADS, 1) tiled_dmma_pass_kernel(const TiledPassArgs a) {
     using C = DmmaCfg<K>;
     constexpr int pitch = C::pitch;
@@ -187,7 +188,7 @@ __global__ void __launch_bounds__(TD_THREADS, 1) tiled_dmma_pass_kernel(const Ti
                     ssum = fma(e0, e0, ssum);
                     ssum = fma(e1, e1, ssum);
                 } else {
-                    dmma_tiles<K, 2, 1, 0>(R, x, vt + off1, vt + off2a, vt + off2b, g, inall, hi_ok);
+                    dmma_tiles<K, 2, 1, 0, DIV>(R, x, vt + off1, vt + off2a, vt + off2b, g, inall, hi_ok);
                 }
                 xp += 8;
                 ++tile;
@@ -232,37 +233,38 @@ __global__ void __launch_bounds__(TD_THREADS, 1) tiled_dmma_pass_kernel(const Ti
     }
 }
 
-template <int K, bool OBJ>
+template <int K, bool OBJ, bool DIV>
 cudaError_t launch_td(const TiledPassArgs& a, cudaStream_t s) {
+    constexpr auto kernel = tiled_dmma_pass_kernel<K, OBJ, DIV>;
     const size_t smem = (size_t)TD_ST * TD_TCH * DmmaCfg<K>::pitch * sizeof(double);
     const long long grid = (long long)a.S * a.nblocks * a.R;
     if (grid > 2147483647ll) return cudaErrorInvalidValue;
-    cudaError_t e = cudaFuncSetAttribute(tiled_dmma_pass_kernel<K, OBJ>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+    cudaError_t e = cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
     if (e != cudaSuccess) return e;
-    tiled_dmma_pass_kernel<K, OBJ><<<(unsigned)grid, TD_THREADS, smem, s>>>(a);
+    kernel<<<(unsigned)grid, TD_THREADS, smem, s>>>(a);
     return cudaGetLastError();
 }
 
-template <bool OBJ>
+template <bool OBJ, bool DIV = false>
 cudaError_t dispatch_td(const TiledPassArgs& a, cudaStream_t s) {
     switch (a.ktmpl) {
-        case 4: return launch_td<4, OBJ>(a, s);
-        case 5: return launch_td<5, OBJ>(a, s);
-        case 6: return launch_td<6, OBJ>(a, s);
-        case 7: return launch_td<7, OBJ>(a, s);
-        case 8: return launch_td<8, OBJ>(a, s);
-        case 9: return launch_td<9, OBJ>(a, s);
-        case 10: return launch_td<10, OBJ>(a, s);
-        case 11: return launch_td<11, OBJ>(a, s);
-        case 12: return launch_td<12, OBJ>(a, s);
-        case 16: return launch_td<16, OBJ>(a, s);
-        case 20: return launch_td<20, OBJ>(a, s);
-        case 24: return launch_td<24, OBJ>(a, s);
-        case 32: return launch_td<32, OBJ>(a, s);
-        case 40: return launch_td<40, OBJ>(a, s);
-        case 48: return launch_td<48, OBJ>(a, s);
-        case 56: return launch_td<56, OBJ>(a, s);
-        case 64: return launch_td<64, OBJ>(a, s);
+        case 4: return launch_td<4, OBJ, DIV>(a, s);
+        case 5: return launch_td<5, OBJ, DIV>(a, s);
+        case 6: return launch_td<6, OBJ, DIV>(a, s);
+        case 7: return launch_td<7, OBJ, DIV>(a, s);
+        case 8: return launch_td<8, OBJ, DIV>(a, s);
+        case 9: return launch_td<9, OBJ, DIV>(a, s);
+        case 10: return launch_td<10, OBJ, DIV>(a, s);
+        case 11: return launch_td<11, OBJ, DIV>(a, s);
+        case 12: return launch_td<12, OBJ, DIV>(a, s);
+        case 16: return launch_td<16, OBJ, DIV>(a, s);
+        case 20: return launch_td<20, OBJ, DIV>(a, s);
+        case 24: return launch_td<24, OBJ, DIV>(a, s);
+        case 32: return launch_td<32, OBJ, DIV>(a, s);
+        case 40: return launch_td<40, OBJ, DIV>(a, s);
+        case 48: return launch_td<48, OBJ, DIV>(a, s);
+        case 56: return launch_td<56, OBJ, DIV>(a, s);
+        case 64: return launch_td<64, OBJ, DIV>(a, s);
         default: return cudaErrorInvalidValue;
     }
 }
@@ -274,7 +276,9 @@ int tiled_dmma_chunk() { return TD_TCH; }
 
 // a.k in 4..64 (smaller k are all-DFMA in the resident formulation and stay on the scalar pass); K = the template K of
 // the combine kernel (tiled_template_k), a.nblocks = ceil(nown / 128), a.D step-contiguous
-cudaError_t launch_tiled_dmma_pass(const TiledPassArgs& a, cudaStream_t s) { return dispatch_td<false>(a, s); }
+cudaError_t launch_tiled_dmma_pass(const TiledPassArgs& a, cudaStream_t s, bool div) {
+    return div ? dispatch_td<false, true>(a, s) : dispatch_td<false>(a, s);
+}
 // objective sums: a = the W-update arguments (D = X^T step-contiguous, U = W, V = H), S = 1
 cudaError_t launch_tiled_dmma_objective(const TiledPassArgs& a, cudaStream_t s) { return dispatch_td<true>(a, s); }
 

@@ -103,7 +103,8 @@ __device__ __forceinline__ float rcp_fast(float p) {
 
 // OBJ = true: objective mode.  Only MMA#1 runs (P = U V^T); the quotient warps accumulate (x - p)^2 instead of dividing,
 // nothing is written back to the factors: replaces tiled_objective_kernel (NMFkMultiplicative.jl:74,125) for Float32.
-template <int K8, int N2, bool OBJ>
+// DIV (pass mode only): the quotient of NMF.jl's KL update (Variant KL_DIV), x / (p + delta); a.den already holds the sums + delta
+template <int K8, int N2, bool OBJ, bool DIV = false>
 __global__ void __launch_bounds__((TcCfg<K8, N2>::THREADS), 1) tc_pass_kernel(const TiledPassArgs a, int* errflag) {
     using C = TcCfg<K8, N2>;
     constexpr int TC_NXS = C::NXS, TC_NVB = C::NVB;
@@ -477,6 +478,12 @@ __global__ void __launch_bounds__((TcCfg<K8, N2>::THREADS), 1) tc_pass_kernel(co
                         // the quotient and the low part: 8 instead of 10 issue slots per pair of elements.
 #pragma unroll
                         for (int j = 0; j < 16; j += 2) {
+                            if constexpr (DIV) {
+                                unsigned long long p2 = pack2(__uint_as_float(p[j]), __uint_as_float(p[j + 1]));
+                                asm("add.rn.f32x2 %0, %1, %2;" : "=l"(p2) : "l"(p2), "l"(pack2(kKlDivDelta<float>, kKlDivDelta<float>)));
+                                p[j] = (uint32_t)p2;
+                                p[j + 1] = (uint32_t)(p2 >> 32);
+                            }
                             const float r0 = rcp_fast(__uint_as_float(p[j])), r1 = rcp_fast(__uint_as_float(p[j + 1]));
                             const unsigned long long x2 = pack2(xh[j * TC_M], xh[(j + 1) * TC_M]), r2 = pack2(r0, r1);
                             unsigned long long q2, l2;
@@ -491,7 +498,7 @@ __global__ void __launch_bounds__((TcCfg<K8, N2>::THREADS), 1) tc_pass_kernel(co
                     } else {  // last chunk of the slice: steps past the end contribute nothing
 #pragma unroll
                         for (int j = 0; j < 16; ++j) {
-                            float q = xh[j * TC_M] * rcp_fast(__uint_as_float(p[j]));
+                            float q = xh[j * TC_M] * rcp_fast(DIV ? __uint_as_float(p[j]) + kKlDivDelta<float> : __uint_as_float(p[j]));
                             q = (jh + half * 16 + j < cnt) ? q : 0.f;
                             const uint32_t h = __float_as_uint(q) & 0xffffe000u;
                             lo[j] = __float_as_uint(q - __uint_as_float(h));
@@ -580,15 +587,16 @@ __global__ void __launch_bounds__((TcCfg<K8, N2>::THREADS), 1) tc_pass_kernel(co
     if (warp == 0) tc::tmem_dealloc<C::TCOLS>(tbase);
 }
 
-template <int K8, int N2, bool OBJ>
+template <int K8, int N2, bool OBJ, bool DIV = false>
 cudaError_t launch_tc(const TiledPassArgs& a, int* d_errflag, cudaStream_t s) {
     using C = TcCfg<K8, N2>;
+    constexpr auto kernel = tc_pass_kernel<K8, N2, OBJ, DIV>;
     const int ngroups = (a.R + C::RB - 1) / C::RB;
     const long long grid = (long long)a.S * a.nblocks * ngroups;
     if (grid > 2147483647ll) return cudaErrorInvalidValue;
-    cudaError_t e = cudaFuncSetAttribute(tc_pass_kernel<K8, N2, OBJ>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)C::SMEM);
+    cudaError_t e = cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)C::SMEM);
     if (e != cudaSuccess) return e;
-    tc_pass_kernel<K8, N2, OBJ><<<(unsigned)grid, C::THREADS, C::SMEM, s>>>(a, d_errflag);
+    kernel<<<(unsigned)grid, C::THREADS, C::SMEM, s>>>(a, d_errflag);
     return cudaGetLastError();
 }
 
@@ -610,8 +618,16 @@ bool tc_pass_supported(const TiledPassArgs& a) {
     return !a.has_nan && a.k >= 1 && a.k <= kTiledMaxK && (a.nown % 4) == 0 && (reinterpret_cast<uintptr_t>(a.D) % 16) == 0;
 }
 
-cudaError_t launch_tc_pass(const TiledPassArgs& a, int* d_errflag, cudaStream_t s) {
-    if (tc2_pass_enabled(a.k)) return launch_tc2_pass(a, d_errflag, s);
+cudaError_t launch_tc_pass(const TiledPassArgs& a, int* d_errflag, cudaStream_t s, bool div) {
+    if (tc2_pass_enabled(a.k)) return launch_tc2_pass(a, d_errflag, s, div);
+    if (div) {
+        if (a.k <= 8) return launch_tc<8, 16, false, true>(a, d_errflag, s);
+        if (a.k <= 16) return launch_tc<16, 16, false, true>(a, d_errflag, s);
+        if (a.k <= 24) return launch_tc<24, 32, false, true>(a, d_errflag, s);
+        if (a.k <= 32) return launch_tc<32, 32, false, true>(a, d_errflag, s);
+        if (a.k <= 48) return launch_tc<48, 64, false, true>(a, d_errflag, s);
+        return launch_tc<64, 64, false, true>(a, d_errflag, s);
+    }
     if (a.k <= 8) return launch_tc<8, 16, false>(a, d_errflag, s);
     if (a.k <= 16) return launch_tc<16, 16, false>(a, d_errflag, s);
     if (a.k <= 24) return launch_tc<24, 32, false>(a, d_errflag, s);

@@ -130,7 +130,8 @@ __global__ void __launch_bounds__(256) tc2_images_kernel(const TiledPassArgs a, 
     }
 }
 
-template <int K8>
+// DIV: the quotient of NMF.jl's KL update (Variant KL_DIV), x / (p + delta); a.den already holds the sums + delta
+template <int K8, bool DIV = false>
 __global__ void __launch_bounds__((Tc2Cfg<K8>::THREADS), 1) tc2_pass_kernel(const TiledPassArgs a, const __grid_constant__ CUtensorMap mX,
                                                                             int* errflag) {
     using C = Tc2Cfg<K8>;
@@ -441,6 +442,12 @@ __global__ void __launch_bounds__((Tc2Cfg<K8>::THREADS), 1) tc2_pass_kernel(cons
                             // per PAIR of quotients, r = 1 / (p0 p1), was measured: no gain - the MUFU pipe is not what bounds this
                             // stage - and p0 p1 underflows for the tiny products of all-zero rows.)
                             const int jj = j;
+                            if constexpr (DIV) {
+                                unsigned long long p2 = pack2f(__uint_as_float(p[jj]), __uint_as_float(p[jj + 1]));
+                                asm("add.rn.f32x2 %0, %1, %2;" : "=l"(p2) : "l"(p2), "l"(pack2f(kKlDivDelta<float>, kKlDivDelta<float>)));
+                                p[jj] = (uint32_t)p2;
+                                p[jj + 1] = (uint32_t)(p2 >> 32);
+                            }
                             const float r0 = rcp_approx(__uint_as_float(p[jj])), r1 = rcp_approx(__uint_as_float(p[jj + 1]));
                             const unsigned long long x2 = pack2f(xv[j], xv[j + 1]), r2 = pack2f(r0, r1);
                             unsigned long long q2, l2;
@@ -456,7 +463,7 @@ __global__ void __launch_bounds__((Tc2Cfg<K8>::THREADS), 1) tc2_pass_kernel(cons
 #pragma unroll
                         for (int j = 0; j < 16; ++j) {
                             const int jj = j;
-                            float q = xv[j] * rcp_approx(__uint_as_float(p[jj]));
+                            float q = xv[j] * rcp_approx(DIV ? __uint_as_float(p[jj]) + kKlDivDelta<float> : __uint_as_float(p[jj]));
                             q = (jh + half * 16 + jj < cnt) ? q : 0.f;
                             const uint32_t h = __float_as_uint(q) & 0xffffe000u;
                             lo[j] = __float_as_uint(q - __uint_as_float(h));
@@ -541,14 +548,15 @@ __global__ void __launch_bounds__((Tc2Cfg<K8>::THREADS), 1) tc2_pass_kernel(cons
     if (warp == 0) tc::tmem_dealloc<C::TCOLS>(tbase);
 }
 
-template <int K8>
+template <int K8, bool DIV>
 cudaError_t launch2(const TiledPassArgs& a, int* d_errflag, cudaStream_t s) {
+    constexpr auto kernel = tc2_pass_kernel<K8, DIV>;
     using C = Tc2Cfg<K8>;
     const int ngroups = (a.R + C::RB - 1) / C::RB;
     const long long grid = (long long)a.S * a.nblocks * ngroups;
     const int chunks = (a.nred + C::TS - 1) / C::TS;
     if (grid > 2147483647ll || a.vimg == nullptr || a.R > 65535) return cudaErrorInvalidValue;
-    cudaError_t e = cudaFuncSetAttribute(tc2_pass_kernel<K8>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)C::SMEM);
+    cudaError_t e = cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)C::SMEM);
     if (e != cudaSuccess) return e;
     // Dstep: element (own o, step t) at Dstep[t + o * nred].  The map is a pure function of (Dstep, nown, nred): the two maps of
     // a solve (X and its transpose) are encoded once and reused by every launch.
@@ -581,7 +589,7 @@ cudaError_t launch2(const TiledPassArgs& a, int* d_errflag, cudaStream_t s) {
     tc2_images_kernel<K8><<<dim3((unsigned)chunks, (unsigned)a.R), 256, 0, s>>>(a, chunks);
     e = cudaGetLastError();
     if (e != cudaSuccess) return e;
-    tc2_pass_kernel<K8><<<(unsigned)grid, C::THREADS, C::SMEM, s>>>(a, mX, d_errflag);
+    kernel<<<(unsigned)grid, C::THREADS, C::SMEM, s>>>(a, mX, d_errflag);
     return cudaGetLastError();
 }
 
@@ -619,9 +627,10 @@ void tc2_pass_prepare() {
     cudaFuncSetAttribute(tc2_pass_kernel<16>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)Tc2Cfg<16>::SMEM);
 }
 
-cudaError_t launch_tc2_pass(const TiledPassArgs& a, int* d_errflag, cudaStream_t s) {
-    if (a.k <= 8) return launch2<8>(a, d_errflag, s);
-    return launch2<16>(a, d_errflag, s);
+cudaError_t launch_tc2_pass(const TiledPassArgs& a, int* d_errflag, cudaStream_t s, bool div) {
+    if (div) return a.k <= 8 ? launch2<8, true>(a, d_errflag, s) : launch2<16, true>(a, d_errflag, s);
+    if (a.k <= 8) return launch2<8, false>(a, d_errflag, s);
+    return launch2<16, false>(a, d_errflag, s);
 }
 
 }  // namespace nmfk

@@ -144,6 +144,15 @@ __host__ __device__ constexpr int resident_threads(int Ktemplate) { return Ktemp
 constexpr int kResidentMaxK = 32;
 constexpr int kTiledMaxK = 64;
 
+// delta of Variant KL_DIV (NMF.jl's MultUpdate(obj=:div)): Q = X ./ (W*H .+ delta), U .*= (numerators) ./ (sums .+ delta) with
+// delta = sqrt(eps(T)), the same (unpinned) reading of NMF.jl as Variant FRO's.  The only place the device takes it from.
+template <typename T>
+constexpr T kKlDivDelta = T(0);
+template <>
+constexpr float kKlDivDelta<float> = 3.4526698e-4f;  // sqrt(eps(Float32)) = 2^-11.5, rounded to Float32
+template <>
+constexpr double kKlDivDelta<double> = 1.4901161193847656e-8;  // sqrt(eps(Float64)) = 2^-26
+
 // template K actually instantiated for a requested k (exact up to 12, then padded)
 inline int resident_template_k(int k) {
     if (k <= 12) return k;

@@ -2,7 +2,7 @@
 #
 # Same signatures and return shapes as the reference for this path
 #   NMFk.NMFmultiplicative   (NMFk.jl/src/NMFkMultiplicative.jl:24, :129 for the distributed method's stop rule)
-#   NMFk.execute_singlerun   (NMFk.jl/src/NMFkExecute.jl:714,729)   method=:simple and method=:nmf, algorithm=:multdiv
+#   NMFk.execute_singlerun   (NMFk.jl/src/NMFkExecute.jl:714,729)   method=:simple and method=:nmf, algorithm=:multdiv / :multmse
 #   NMFk.execute_run         (NMFk.jl/src/NMFkExecute.jl:483)
 #   NMFk.execute             (NMFk.jl/src/NMFkExecute.jl:178, 236)  including the JLD result cache (load / save / loadonly)
 #   NMFk.robustkmeans        (NMFk.jl/src/NMFkCluster.jl:138, 172)
@@ -52,12 +52,13 @@ end
 function makeparams(; tol=1e-19, tolOF=1e-3, weight=1, maxiter=10000, maxbaditers=10, maxreattempts=2, stopconv=1000, Wfixed=false, Hfixed=false, normalize=1, engine=0, clusterWmatrix=false, stop_rule=0, method::Symbol=:simple, algorithm::Symbol=:multdiv, kw...)
 	variant = 0
 	if method == :nmf
-		algorithm == :multdiv || error("NMFkB200: method=:nmf covers algorithm=:multdiv (NMF.MultUpdate(obj=:mse)) only")
-		variant = 1
+		# the reference swaps the names (NMFkExecute.jl:765-768): :multdiv = MultUpdate(obj=:mse), :multmse = MultUpdate(obj=:div)
+		algorithm in (:multdiv, :multmse) || error("NMFkB200: method=:nmf covers algorithm=:multdiv and :multmse (NMF.MultUpdate) only")
+		variant = algorithm == :multdiv ? 1 : 3
 	elseif method == :sparsity
 		variant = 2 # NMFsparsity (NMFkSparsity.jl); its own options travel through setsparsity! (called by the entry points)
 	elseif method != :simple
-		error("NMFkB200 covers method=:simple, :sparsity and :nmf with algorithm=:multdiv; use NMFk for $(method)")
+		error("NMFkB200 covers method=:simple, :sparsity and :nmf with algorithm=:multdiv or :multmse; use NMFk for $(method)")
 	end
 	w = typeof(weight) <: Number ? weight : 1 # array weights are installed on the context (setweight!)
 	return Params(tol, tolOF, eps(Float64), w, maxiter, maxbaditers, maxreattempts, stopconv, 10, Wfixed, Hfixed, normalize, 0, engine, clusterWmatrix, stop_rule, variant, 0)

@@ -327,10 +327,14 @@ def _params_from_kw(kw: dict, ctx: Optional[Context] = None, **defaults) -> Para
     vals = dict(defaults)
     method = str(kw.pop("method", "simple")).lstrip(":")
     algorithm = str(kw.pop("algorithm", "multdiv")).lstrip(":")
-    if method == "nmf":  # NMFkExecute.jl:763-775: NMF.jl solvers; :multdiv is MultUpdate(obj=:mse) = Variant FRO
-        if algorithm != "multdiv":
-            raise NMFkError(-6, "method=:nmf: only algorithm=:multdiv (NMF.MultUpdate(obj=:mse)) is on the B200 path")
-        vals["variant"] = 1
+    if method == "nmf":  # NMFkExecute.jl:763-775: NMF.jl solvers, names swapped in the reference (:765-768):
+        # :multdiv is MultUpdate(obj=:mse) = Variant FRO, :multmse is MultUpdate(obj=:div) = Variant KL_DIV
+        if algorithm == "multdiv":
+            vals["variant"] = 1
+        elif algorithm == "multmse":
+            vals["variant"] = 3
+        else:
+            raise NMFkError(-6, "method=:nmf: only algorithm=:multdiv and :multmse (NMF.MultUpdate) are on the B200 path")
     elif method == "sparsity":  # NMFkExecute.jl:757-758: NMFsparsity(Xn, nk; maxiter, tol, kw...)
         if ctx is None:
             raise NMFkError(-1, "method=:sparsity needs a context")
@@ -342,7 +346,8 @@ def _params_from_kw(kw: dict, ctx: Optional[Context] = None, **defaults) -> Para
               ctx._h)
         vals["variant"] = 2
     elif method != "simple":
-        raise NMFkError(-6, "method=:%s is not on the B200 path (:simple, :sparsity and :nmf with algorithm=:multdiv are)" % method)
+        raise NMFkError(-6, "method=:%s is not on the B200 path (:simple, :sparsity and :nmf with algorithm=:multdiv or :multmse "
+                            "are)" % method)
     for k in list(kw):
         if k in _PARAM_NAMES:
             vals[k] = kw.pop(k)
